@@ -3,7 +3,7 @@
 with lexifair assignment), BASELINE.json config 2: 3 agents / 3 goals / 3 obstacles, FA+FR reward,
 goal_rew = collision_rew = 30, episode_length 25, 65 536 envs per B200, random actions.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1; envs sharded by global env index, weak scaling: 65 536
 envs per GPU).  Prints ONE JSON line on rank 0.  A "step" is one env step of the whole batch.
@@ -17,7 +17,7 @@ envs per GPU).  Prints ONE JSON line on rank 0.  A "step" is one env step of the
   env-step) / average step-kernel duration from CUDA events, against MEASURED_PEAKS.json hbm_gbs.
 * ``cpu_baseline``  the numpy oracle port (oracle/navgraph.py) on all host cores, bounded sample.
 * ``--impl reference``  times that CPU port as the reference arm (the reference itself is pure Python that
-  needs /root/reference, which does not exist on the GPU box; the port is pinned to it by tests/golden).
+  needs a checkout of the original project, which this repository does not contain; the port is pinned to it by tests/golden).
 """
 from __future__ import annotations
 
@@ -81,6 +81,28 @@ def lookup_traffic(table: dict, kernel_name: str, envs_per_gpu: int, walls: int)
     """dram__bytes_read.sum + dram__bytes_write.sum per launch of the ncu capture that matches this run, else None."""
     ent = lookup_traffic_entry(table, kernel_name, envs_per_gpu, walls)
     return ent.get("dram_bytes_per_launch") if ent else None
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, per_env: dict, whole: dict) -> None:
+    """``--dump-outputs``: write every array as ``path/<name>.npy`` (float64 stays float64, the rest becomes float32).
+    ``per_env`` arrays have the env index first; if all arrays together exceed DUMP_LIMIT_BYTES, every per-env array
+    keeps the same env rows: a sample drawn with a fixed seed from the batch size alone, in ascending env order."""
+    import numpy as np
+    as_float = lambda a: np.asarray(a, dtype=np.float64 if a.dtype == np.float64 else np.float32)
+    per_env = {k: as_float(v) for k, v in per_env.items()}
+    whole = {k: as_float(v) for k, v in whole.items()}
+    B = next(iter(per_env.values())).shape[0]
+    row_bytes = sum(v.nbytes // B for v in per_env.values())
+    room = DUMP_LIMIT_BYTES - sum(v.nbytes for v in whole.values()) - 4096        # 4096: the .npy headers
+    if row_bytes * B > room:
+        rows = np.sort(np.random.default_rng(0).choice(B, room // row_bytes, replace=False))
+        per_env = {k: v[rows] for k, v in per_env.items()}
+    os.makedirs(path, exist_ok=True)
+    for name, a in {**per_env, **whole}.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def sim_kwargs():
@@ -211,8 +233,7 @@ def cpu_port_throughput(steps: int, warm: int, envs_per_proc: int = 2048, config
 def run_reference(args, rank: int, world: int):
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 200))
-    warm = max(1, min(args.warmup, 25))
+    steps, warm = args.steps, max(0, args.warmup)
     value, cores, sample, ms = cpu_port_throughput(steps, warm, config=args.config)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "agent-steps/s", "n_gpus": args.gpus,
@@ -252,7 +273,7 @@ def run_rollout(args, rank: int, local_rank: int, world: int):
     col = fm.RolloutCollector(env, actor, critic, max_graphs=args.max_graphs,
                               generator=torch.Generator(device=dev).manual_seed(1234 + rank))
     col.warmup()
-    episodes = max(1, args.steps // EPISODE)
+    episodes = args.steps // EPISODE               # main() admits whole episodes only
     K = episodes * EPISODE
     col.run()                                       # warm-up episode (allocator, library handles)
     col.buffer.after_update()
@@ -565,6 +586,11 @@ def run_ours(args, rank: int, local_rank: int, world: int):
         elapsed_ms = float(tt.item())
     value = B * world * N_AGENTS * K / (elapsed_ms * 1e-3)
     total_stats = stats.summary()
+    if args.dump_outputs and rank == 0:          # before the closed-loop and e2e steps below overwrite the slab ring
+        last = env.slot_outputs(env._slot)       # the slab the last timed step wrote
+        dump_outputs(args.dump_outputs,
+                     {k: last[k].cpu().numpy() for k in ("obs", "node_obs", "adj_env", "reward", "done", "info")},
+                     {"episode_stats": stats.result().cpu().numpy()})
 
     # roofline of the step kernel: algorithmic bytes per launch / average launch duration
     peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
@@ -731,7 +757,17 @@ def main():
                          "regions keep a deep eager launch queue anyway (measured: 0.93 eager vs 0.87 replayed at 5000 steps), "
                          "and the group mapping's next-episode prefetch is a host-side decision that a replay cannot make")
     ap.add_argument("--no-step-graph", dest="step_graph", action="store_const", const="off")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (obs, node_obs, adj_env, reward, done, "
+                         "info; a fixed env sample if above 64 MB) and the episode statistics as DIR/<name>.npy (rank 0); "
+                         "configs c1-c4")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.config == "c5" and args.impl == "ours" and args.steps % EPISODE:
+        ap.error(f"--config c5 times whole episodes: --steps must be a multiple of {EPISODE}")
+    if args.dump_outputs and (args.impl == "reference" or args.config in ("c5", "form")):
+        ap.error("--dump-outputs covers the step configs c1-c4 of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -19,8 +19,8 @@ What is here
 * ``edges.py``      the policy-side edge list (``process_adj``) restated.
 * ``pyg_stub.py``   stand-in for the torch_geometric primitives the reference policy uses, so that the reference's own
   ``GR_Actor`` / ``GR_Critic`` run here as the checker of ``fair_marl_b200.policy`` (``make_policy_golden.py``).
-* ``reference_shim.py`` imports the UNMODIFIED reference from ``/root/reference``
-  (only in the build container, where it exists) to pin the restatement and to
+* ``reference_shim.py`` imports the UNMODIFIED reference from the checkout named by
+  ``FAIRMARL_REFERENCE_ROOT`` (only where that is set) to pin the restatement and to
   generate ``tests/golden/*.npz`` (``make_golden.py``).
 
 Parity pinning

@@ -4,7 +4,7 @@ Reference: ``marl_fair_assign.py:16-55`` (``solve_fair_assignment``), called
 from ``multiagent/custom_scenarios/navigation_graph.py:555-561``.
 
 The reference solves n rounds of a binary MILP with pyomo + ``gurobi_persistent``
-(neither vendored under /root/reference nor installable here; requirements.txt:2
+(neither vendored in the original project nor installable here; requirements.txt:2
 pins gurobipy==10.0.2, pyomo is unpinned).  Round k: minimise z subject to
 ``cost_helper[i,j] * x[i,j] <= z`` over perfect matchings x, with the rows fixed
 in earlier rounds held; then the entry of ``costs`` closest to the optimum z is

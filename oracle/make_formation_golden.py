@@ -1,4 +1,4 @@
-"""Record formation-family fixtures from the UNMODIFIED reference (build container only; TEST INFRASTRUCTURE).
+"""Record formation-family fixtures from the UNMODIFIED reference (needs FAIRMARL_REFERENCE_ROOT; TEST INFRASTRUCTURE).
 
     python -m oracle.make_formation_golden            # writes tests/golden/formation_*.npz
 

@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference (TEST INFRASTRUCTURE ONLY).
 
-Run in the build container (needs /root/reference):
+Run with FAIRMARL_REFERENCE_ROOT set to a checkout of the original project:
 
-    python -m oracle.make_golden
+    FAIRMARL_REFERENCE_ROOT=<checkout> python -m oracle.make_golden
 
 For every config a single reference ``MultiAgentGraphEnv`` (built exactly as
 multiagent/MPE_env.py:62-75 builds it, with the two stubs of

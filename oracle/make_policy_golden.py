@@ -1,4 +1,4 @@
-"""Golden vectors for the dense graph policy (TEST INFRASTRUCTURE ONLY; run in the build container).
+"""Golden vectors for the dense graph policy (TEST INFRASTRUCTURE ONLY; needs FAIRMARL_REFERENCE_ROOT).
 
 Builds the UNMODIFIED reference ``GR_Actor`` / ``GR_Critic`` (onpolicy/algorithms/graph_actor_critic.py) on top of
 the ``gym`` stub (reference_shim) and the torch_geometric stand-in (pyg_stub), feeds them seeded inputs shaped like

@@ -2,7 +2,7 @@
 over envs (TEST INFRASTRUCTURE ONLY -- see oracle/__init__.py).
 
 Every function cites the reference lines it follows (paths relative to
-/root/reference).  Arithmetic is float64 in the reference's own operation order,
+the original project's root).  Arithmetic is float64 in the reference's own operation order,
 so that this file agrees with the imported reference to ~1e-13
 (tests/test_oracle_vs_golden.py pins it against tests/golden/*.npz, which were
 produced by running the UNMODIFIED reference: oracle/make_golden.py).

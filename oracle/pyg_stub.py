@@ -1,7 +1,7 @@
 """Minimal stand-in for ``torch_geometric`` (TEST INFRASTRUCTURE ONLY, "parity unpinned" w.r.t. PyG).
 
 The reference's policy (``onpolicy/algorithms/utils/gnn_new.py``, legacy twin ``gnn.py``) is built on
-torch_geometric, which is not installed here and not vendored under ``/root/reference``
+torch_geometric, which is not installed here and not vendored in the original project
 (requirements.txt pins ``torch_geometric==2.3.1``).  To run the reference's OWN ``GNNBase`` /
 ``GR_Actor`` / ``GR_Critic`` code as the checker of ``fair_marl_b200.policy`` this module restates, on
 edge lists with gather / index_add, the few published PyG primitives those files use:

@@ -1,7 +1,7 @@
 """The reference's own CPU path, timed as SURVEY.md section 8(d) / BASELINE.md section 3 specify: the UNMODIFIED
 ``GraphSubprocVecEnv`` (onpolicy/envs/env_wrappers.py:951-1025) over the unmodified ``GraphMPEEnv`` / ``MultiAgentGraphEnv`` +
 ``navigation_graph.Scenario``, one worker process per env, random one-hot actions, episode_length 25 with auto-reset.
-TEST / MEASUREMENT INFRASTRUCTURE ONLY; needs /root/reference (build container), so it cannot run on the GPU box: its
+TEST / MEASUREMENT INFRASTRUCTURE ONLY; needs the original project's checkout (FAIRMARL_REFERENCE_ROOT), not a GPU: its
 JSON lines are committed under profiles/ next to the port's numbers (bench.py cpu_baseline, kind "port").
 
 Gurobi / pyomo are not installable (requirements.txt:2), so the assignment solver is stubbed and the stub is stated:

@@ -1,7 +1,7 @@
 """Import the UNMODIFIED reference env as a checker (TEST INFRASTRUCTURE ONLY).
 
-Only usable where ``/root/reference`` exists (the build container); the GPU box
-does not have it, so nothing in ``-m gpu`` tests / smoke / bench imports this.
+Only usable where ``FAIRMARL_REFERENCE_ROOT`` names a checkout of the original Fair-MARL
+project, which this repository does not contain; nothing in ``-m gpu`` tests / smoke / bench imports this.
 Recipe: SURVEY.md Appendix A -- stub ``gym`` (absent) and ``marl_fair_assign``
 (needs pyomo + gurobi) in ``sys.modules``, load the scenario file by path
 (``custom_scenarios/__init__.py`` uses the removed ``imp`` module), and wire the
@@ -20,11 +20,12 @@ import numpy as np
 from . import lexifair
 from .navgraph import NavConfig, NavState
 
-REFERENCE_ROOT = os.environ.get("FAIRMARL_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("FAIRMARL_REFERENCE_ROOT", "")
+SKIP_REASON = "needs the original Fair-MARL project: set FAIRMARL_REFERENCE_ROOT to its checkout"
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "multiagent", "core.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "multiagent", "core.py"))
 
 
 def _mod(name, **kw):

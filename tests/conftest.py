@@ -11,7 +11,7 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs the original Fair-MARL project (FAIRMARL_REFERENCE_ROOT)")
 
 
 def pytest_generate_tests(metafunc):
@@ -41,9 +41,9 @@ def _gpu_ready() -> bool:
 
 
 def pytest_collection_modifyitems(config, items):
-    from oracle.reference_shim import reference_available
+    from oracle.reference_shim import SKIP_REASON, reference_available
     have_ref, have_gpu = reference_available(), _gpu_ready()
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
+    skip_ref = pytest.mark.skip(reason=SKIP_REASON)
     skip_gpu = pytest.mark.skip(reason="no CUDA device (or libfairmarl.so not built): GPU parity tests run on the B200 box")
     for item in items:
         if not have_ref and "reference" in item.keywords:

@@ -68,21 +68,31 @@ def test_library_is_sm100a_only(lib_path):
     assert "sm_100a" in out and "sm_90" not in out and "sm_80" not in out
 
 
+_NO_CPU_FALLBACK = """
+import ctypes
+import fair_marl_b200
+from fair_marl_b200 import _lib
+try:
+    fair_marl_b200.B200GraphVecEnv(fair_marl_b200.SimConfig(), num_envs=4)
+    raise SystemExit("B200GraphVecEnv was created without a CUDA device")
+except _lib.FairMarlError:
+    pass
+# the C entry point itself reports "no device" instead of computing anything
+lib = _lib.load()
+cfg = _lib.FmConfig(num_envs=4, num_agents=3, num_obstacles=3, episode_length=25)
+h = ctypes.c_void_p()
+rc = lib.fm_create(ctypes.byref(cfg), 0, ctypes.byref(h))
+assert rc == -4 and b"no CUDA device" in lib.fm_last_error(), (rc, lib.fm_last_error())
+"""
+
+
 def test_no_cpu_fallback(lib_path):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    import fair_marl_b200
-    from fair_marl_b200._lib import FairMarlError
-    with pytest.raises(FairMarlError):
-        fair_marl_b200.B200GraphVecEnv(fair_marl_b200.SimConfig(), num_envs=4)
-    # the C entry point itself reports "no device" instead of computing anything
-    from fair_marl_b200 import _lib
-    lib = _lib.load()
-    cfg = _lib.FmConfig(num_envs=4, num_agents=3, num_obstacles=3, episode_length=25)
-    h = ctypes.c_void_p()
-    rc = lib.fm_create(ctypes.byref(cfg), 0, ctypes.byref(h))
-    assert rc == -4 and b"no CUDA device" in lib.fm_last_error()
+    """Runs in a child process that sees no CUDA device, so the check holds on GPU machines too."""
+    import subprocess
+    import sys
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    res = subprocess.run([sys.executable, "-c", _NO_CPU_FALLBACK], cwd=ROOT, env=env, capture_output=True, text=True)
+    assert res.returncode == 0, res.stdout + res.stderr
 
 
 def test_invalid_config_is_rejected(lib_path):
@@ -190,13 +200,44 @@ def test_integration_doc_formation_stub_matches_binding():
     assert [(n, getattr(C, t)) for n, t in doc_fields] == list(_lib.FmFormationConfig._fields_)
 
 
-def test_bench_reports_ncu_traffic_only_for_the_matching_kernel():
-    """roofline.traffic comes from the ncu capture of the SAME kernel at the SAME size (profiles/step_kernel_traffic.json)."""
+def _load_bench():
     import importlib.util
-    import json
     spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_dump_outputs_is_float_bounded_and_reproducible(tmp_path, monkeypatch):
+    import numpy as np
+    bench = _load_bench()
+    B = 1000
+    rng = np.random.default_rng(1)
+    per_env = {"obs": rng.random((B, 3, 7), dtype=np.float32), "done": rng.integers(0, 2, (B, 3)).astype(np.uint8)}
+    whole = {"episode_stats": rng.random(47)}
+    bench.dump_outputs(str(tmp_path / "full"), per_env, whole)
+    got = {p.stem: np.load(p) for p in (tmp_path / "full").iterdir()}
+    assert sorted(got) == ["done", "episode_stats", "obs"]
+    assert got["obs"].dtype == np.float32 and got["done"].dtype == np.float32 and got["episode_stats"].dtype == np.float64
+    assert np.array_equal(got["obs"], per_env["obs"]) and np.array_equal(got["done"], per_env["done"])
+    limit = 20000
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", limit)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), per_env, whole)
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    b = {p.stem: np.load(p) for p in (tmp_path / "b").iterdir()}
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= limit
+    assert 0 < a["obs"].shape[0] < B and a["obs"].shape[0] == a["done"].shape[0]
+    rows = [int(np.flatnonzero((per_env["obs"] == r).all(axis=(1, 2)))[0]) for r in a["obs"]]
+    assert rows == sorted(rows) and np.array_equal(a["done"], per_env["done"][rows])      # same env rows in every array
+    assert all(np.array_equal(a[k], b[k]) for k in a)                                      # the same sample every run
+    assert np.array_equal(a["episode_stats"], whole["episode_stats"])
+
+
+def test_bench_reports_ncu_traffic_only_for_the_matching_kernel():
+    """roofline.traffic comes from the ncu capture of the SAME kernel at the SAME size (profiles/step_kernel_traffic.json)."""
+    import json
+    bench = _load_bench()
     table = json.load(open(os.path.join(ROOT, "profiles", "step_kernel_traffic.json")))
     assert bench.lookup_traffic(table, "fm::aw_kernel<3,3,0> (agent-warp)", 65536, 0) == 13900800
     c3 = bench.lookup_traffic(table, "fm::step_kernel<8> (group-per-env)", 262144, 0)

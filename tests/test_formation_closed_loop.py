@@ -2,8 +2,8 @@
 reference SHIPS (model_weights/{FA+FR,FA,OA,RA}/actor.pt, trained on the formation scenarios) are loaded into
 fair_marl_b200's dense GNN policy and drive the formation oracle in closed loop.  If any piece of the interface were off --
 the 11-dim observation, the 13-dim node rows, adj, the agent-id gather, the 0..4 action convention, the per-scenario goal
-semantics -- a trained policy would do no better than random moves.  Build container only (the weights live in
-/root/reference)."""
+semantics -- a trained policy would do no better than random moves.  Needs the original project's checkout (the weights live
+there): FAIRMARL_REFERENCE_ROOT."""
 import os
 
 import numpy as np

@@ -1,5 +1,5 @@
 """Pin the numpy oracle against golden vectors produced by the UNMODIFIED reference
-(oracle/make_golden.py, run in the build container)."""
+(oracle/make_golden.py, run against a checkout of it)."""
 import numpy as np
 import pytest
 

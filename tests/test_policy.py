@@ -1,9 +1,9 @@
 """Dense graph policy (fair_marl_b200.policy) vs the reference's GR_Actor / GR_Critic.
 
-* golden: outputs of the UNMODIFIED reference policy code (run in the build container on the torch_geometric
+* golden: outputs of the UNMODIFIED reference policy code (run from its checkout on the torch_geometric
   stand-in, oracle/make_policy_golden.py) -- state dict, inputs and outputs frozen in tests/golden/policy_*.npz;
-* live (only where /root/reference exists): fresh random configurations against the reference modules, and the
-  shipped ``model_weights/*/actor.pt`` (legacy gnn.py key layout) loaded strictly.
+* live (``-m reference``, only where FAIRMARL_REFERENCE_ROOT names the original project's checkout): fresh random
+  configurations against the reference modules, and the shipped ``model_weights/*/actor.pt`` (legacy gnn.py key layout) loaded strictly.
 Tolerance: 1e-5 * max(|ref|, 1) on float32 outputs (the contract of north_star); actions (argmax) exact.
 """
 import ast
@@ -81,7 +81,7 @@ def test_sampling_is_a_valid_categorical_draw():
     assert lp.shape == (M, 1) and torch.all(lp <= 0) and h.shape == (M, 1, 64)
 
 
-needs_reference = pytest.mark.skipif(not reference_shim.reference_available(), reason="/root/reference not present")
+needs_reference = pytest.mark.reference
 
 
 @needs_reference

@@ -1,9 +1,9 @@
-"""Drop-in proof with the reference's OWN runner (SURVEY.md section 8b / 8d C5; build container only).
+"""Drop-in proof with the reference's OWN runner (SURVEY.md section 8b / 8d C5; needs FAIRMARL_REFERENCE_ROOT).
 
 The unmodified ``GMPERunner`` (onpolicy/runner/shared/graph_mpe_runner.py) is instantiated on top of what
 ``B200GraphVecEnv`` returns -- ``tests/golden/b200_vec_env_tuples.npz``, the reset 4-tuple and step 7-tuples recorded
-from the device env on a B200 by tools/record_vec_env_tuples.py (the GPU box has no /root/reference and the build
-container has no GPU, so the hand-over is a recording) -- behind the same spaces object the device env builds
+from the device env on a B200 by tools/record_vec_env_tuples.py (the original project runs on the CPU from its own
+checkout, so the hand-over is a recording) -- behind the same spaces object the device env builds
 (``fair_marl_b200.vec_env.make_spaces``).  Then, with the reference's own code and nothing of ours in between:
 ``warmup`` (:178-203) -> per step ``collect`` (:396-436, the reference's GR_Actor / GR_Critic on its GraphReplayBuffer
 slabs) -> ``envs.step(actions_env)`` -> the data tuple of ``run`` (:60-80) -> ``insert`` (:438-488), and finally

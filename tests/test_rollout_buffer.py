@@ -1,6 +1,6 @@
 """DeviceRolloutBuffer (plain torch, here on the CPU device) vs the reference's GraphReplayBuffer fed through the
 reference's GMPERunner.insert logic (graph_mpe_runner.py:438-488, restated below line by line because GMPERunner
-itself needs a trainer / tensorboard).  Needs /root/reference (skipped on the GPU box)."""
+itself needs a trainer / tensorboard).  Needs the original project's checkout (FAIRMARL_REFERENCE_ROOT)."""
 from argparse import Namespace
 
 import numpy as np
@@ -10,7 +10,7 @@ import torch
 from fair_marl_b200.rollout import DeviceRolloutBuffer
 from oracle import reference_shim
 
-pytestmark = pytest.mark.skipif(not reference_shim.reference_available(), reason="/root/reference not present")
+pytestmark = pytest.mark.reference
 
 
 def _reference_buffer(T, B, N, E, H):

@@ -1,6 +1,6 @@
 """Record what ``B200GraphVecEnv`` hands to the runner -- the reset 4-tuple and a few step 7-tuples, exactly as returned
 (shapes, dtypes, the infos sequence) -- for tests/test_reference_runner.py, which replays them through the UNMODIFIED
-GMPERunner in the build container (/root/reference is not on the GPU box; no GPU in the container).
+GMPERunner from a checkout of the original project (FAIRMARL_REFERENCE_ROOT), which needs no GPU.
 usage (GPU box): python tools/record_vec_env_tuples.py gpurun_out/b200_vec_env_tuples.npz"""
 import os
 import sys
