@@ -143,6 +143,8 @@ def load():
         "fm_formation_step_many": ([vp, vp, i32, C.POINTER(FmOutputs), vp], C.c_int),
         "fm_formation_set_state": ([vp, C.POINTER(FmFormationState), vp], C.c_int),
         "fm_formation_get_state": ([vp, C.POINTER(FmFormationState), vp], C.c_int),
+        "fm_formation_stats_enable": ([vp, i32, vp], C.c_int),
+        "fm_formation_stats_read": ([vp, vp, i32, vp], C.c_int),
         "fm_gnn_weight_floats": ([C.POINTER(FmGnnConfig)], i64),
         "fm_gnn_supported": ([i32, i32], C.c_int),
         "fm_gnn_forward": ([C.c_int, C.POINTER(FmGnnConfig), vp, vp, vp, vp, vp, vp], C.c_int),
@@ -163,7 +165,7 @@ EXPORTED_SYMBOLS = (
     "fm_algorithmic_bytes_per_step", "fm_kernel_launches",
     "fm_formation_create", "fm_formation_destroy", "fm_formation_reset", "fm_formation_step", "fm_formation_step_many",
     "fm_formation_set_state",
-    "fm_formation_get_state", "fm_gnn_weight_floats", "fm_gnn_supported", "fm_gnn_forward",
+    "fm_formation_get_state", "fm_formation_stats_enable", "fm_formation_stats_read", "fm_gnn_weight_floats", "fm_gnn_supported", "fm_gnn_forward",
     "fm_head_weight_floats", "fm_policy_head",
 )
 

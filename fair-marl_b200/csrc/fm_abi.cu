@@ -915,6 +915,9 @@ struct FmFormation {
   cudaEvent_t lane_fork, lane_join;
   fm::FormAsync lane_async;  // the second lane's own prefetch stream / events
   bool has_lane;
+  double* stats;             // episode statistics (allocated on first fm_formation_stats_enable): [ceil(B / 32)][K] partial
+  float* stats_info;         // sums, followed by [B, N, 14] info rows for the steps whose caller passes no info array
+  int stats_rows, K;
 };
 
 // the 23 members of FmFormationState, in declaration order: (words per env, element size)
@@ -948,6 +951,7 @@ int fm_formation_create(const FmFormationConfig* cfg, int device, FmFormation** 
   FmFormation* h = new (std::nothrow) FmFormation();
   if (!h) return fail(FM_ERR_CUDA, "fm_formation_create: out of host memory");
   h->cfg = *cfg; h->device = device; h->has_lane = false;
+  h->stats = nullptr; h->stats_info = nullptr; h->stats_rows = (cfg->num_envs + 31) / 32; h->K = fm_stats_len(cfg->num_agents);
   fm::FormParams& p = h->p;
   memset(&p, 0, sizeof(p));
   p.B = cfg->num_envs; p.N = cfg->num_agents; p.O = cfg->num_obstacles; p.episode_length = cfg->episode_length;
@@ -1005,6 +1009,7 @@ int fm_formation_destroy(FmFormation* h) {
     cudaEventDestroy(h->lane_fork); cudaEventDestroy(h->lane_join); cudaStreamDestroy(h->lane_stream);
     if (h->has_async) { cudaEventDestroy(h->lane_async.fork); cudaEventDestroy(h->lane_async.join); cudaStreamDestroy(h->lane_async.side); }
   }
+  cudaFree(h->stats);
   cudaFree(h->block);
   delete h;
   return FM_OK;
@@ -1019,17 +1024,25 @@ int fm_formation_reset(FmFormation* h, const uint8_t* mask, const FmOutputs* out
   return FM_OK;
 }
 
+// The step's outputs: with statistics on, info rows always go somewhere (the handle's own rows when the caller passes none),
+// so that the statistics do not depend on which outputs the caller asks for.
+static FmOutputs formation_outputs(const FmFormation* h, const FmOutputs& out) {
+  FmOutputs o = out;
+  if (h->p.stats && !o.info) o.info = h->stats_info;
+  return o;
+}
+
 int fm_formation_step(FmFormation* h, const int32_t* actions, const FmOutputs* out, void* stream) {
   if (!h || !actions || !out) return fail(FM_ERR_INVALID_ARG, "fm_formation_step: null argument");
   if (int rc = use_device(h->device)) return rc;
   fm::FormParams p = h->p;
-  p.out = *out; p.actions = actions; p.mask = nullptr;
+  p.out = formation_outputs(h, *out); p.actions = actions; p.mask = nullptr;
   FM_CUDA(fm::launch_formation(p, false, (cudaStream_t)stream, h->has_async ? &h->async : nullptr));
   return FM_OK;
 }
 
 // The handle's launch parameters restricted to envs [start, start + count) (start a multiple of 32): every per-env pointer
-// moves by its own stride, the Philox key by `start`; tile-indexed blocks (recipes, ready flags) by whole tiles.
+// moves by its own stride, the Philox key by `start`; tile-indexed blocks (recipes, ready flags, statistics rows) by whole tiles.
 static fm::FormParams formation_slice(const FmFormation* h, int start, int count, const FmOutputs& out, const int32_t* actions) {
   fm::FormParams p = h->p;
   const size_t B = (size_t)h->p.B;
@@ -1037,7 +1050,7 @@ static fm::FormParams formation_slice(const FmFormation* h, int start, int count
   for (int k = 0; k < 23; ++k)
     if (member[k]) member[k] = (char*)member[k] + h->field_bytes[k] / B * (size_t)start;
   const size_t N = (size_t)p.N, E = 2 * N + (size_t)p.O + (size_t)p.W;
-  p.out = out;
+  p.out = formation_outputs(h, out);
   if (p.out.obs) p.out.obs += (size_t)start * N * FM_FORMATION_OBS_DIM;
   if (p.out.node_obs) p.out.node_obs += (size_t)start * N * E * FM_FORMATION_NODE_FEAT_DIM;
   if (p.out.adj) p.out.adj += (size_t)start * E * E;
@@ -1051,6 +1064,7 @@ static fm::FormParams formation_slice(const FmFormation* h, int start, int count
   if (p.rec) p.rec += fm::formation_recipe_floats(p.N, p.O, start);
   if (p.ready) p.ready += 2 * (start / 32);
   if (p.pend) p.pend += start;                          // SoA: the field stride stays the handle's Bp
+  if (p.stats) p.stats += (size_t)(start / 32) * h->K;
   return p;
 }
 
@@ -1108,6 +1122,31 @@ int fm_formation_set_state(FmFormation* h, const FmFormationState* st, void* str
 
 int fm_formation_get_state(FmFormation* h, const FmFormationState* st, void* stream) {
   return formation_state_copy(h, st, false, stream, "fm_formation_get_state");
+}
+
+int fm_formation_stats_enable(FmFormation* h, int32_t enable, void* stream) {
+  if (!h) return fail(FM_ERR_INVALID_ARG, "fm_formation_stats_enable: null argument");
+  if (int rc = use_device(h->device)) return rc;
+  if (enable && !h->stats) {
+    const size_t rows = (size_t)h->stats_rows * h->K * sizeof(double);
+    const size_t info = (size_t)h->p.B * h->p.N * FM_INFO_DIM * sizeof(float);
+    void* block = nullptr;
+    FM_CUDA(cudaMalloc(&block, rows + info));
+    cudaError_t e = cudaMemsetAsync(block, 0, rows + info, (cudaStream_t)stream);
+    if (e != cudaSuccess) { cudaFree(block); return fail(FM_ERR_CUDA, "fm_formation_stats_enable: %s", cudaGetErrorString(e)); }
+    h->stats = (double*)block;
+    h->stats_info = (float*)((char*)block + rows);
+  }
+  h->p.stats = enable ? h->stats : nullptr;
+  return FM_OK;
+}
+
+int fm_formation_stats_read(FmFormation* h, double* out_dev, int32_t clear, void* stream) {
+  if (!h || !out_dev) return fail(FM_ERR_INVALID_ARG, "fm_formation_stats_read: null argument");
+  if (!h->p.stats) return fail(FM_ERR_INVALID_ARG, "fm_formation_stats_read: episode statistics are off (fm_formation_stats_enable)");
+  if (int rc = use_device(h->device)) return rc;
+  FM_CUDA(fm::launch_stats_reduce(h->stats, h->stats_rows, h->K, out_dev, clear, (cudaStream_t)stream));
+  return FM_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------------

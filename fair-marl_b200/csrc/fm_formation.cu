@@ -139,6 +139,45 @@ __device__ void form_emit(const FormParams& p, float* __restrict__ S, const Form
   if (lane == 0) bulk_wait_read<0>();
 }
 
+// Episode statistics of one step into the warp's own row of p.stats (layout of fm_stats_read): per agent the emitted reward,
+// per agent the 14 info values of the envs whose agents are all done, the number of those envs and the env-steps.  Lane =
+// env; reward and done come from the warp's images, info from the row this lane has just written.  Lanes >= nenv add 0.
+// Only lane 0 adds into the row and only this warp owns it, so the order of the adds is fixed: the sums are deterministic
+// (reductions from one thread to one address are performed in program order).
+// A global-space reduction: fire-and-forget.  Through the generic atomicAdd(double*) the compiler emits a returning ATOM
+// behind a shared-memory CAS-loop branch here (it cannot see that p.stats is global), and lane 0 waits for every result.
+__device__ __forceinline__ void red_add(double* a, double v) {
+  asm volatile("red.global.add.f64 [%0], %1;" :: "l"(__cvta_generic_to_global(a)), "d"(v) : "memory");
+}
+
+template <int N>
+__device__ __forceinline__ void form_stats(const FormParams& p, const float* S, const FormTile& t, int env0, int nenv, int lane) {
+  double* row = p.stats + (size_t)(env0 >> 5) * (15 * N + 2);
+  const bool live = lane < nenv;
+  const uint8_t* done = reinterpret_cast<const uint8_t*>(S + t.done) + lane * N;
+  bool all_done = live;
+#pragma unroll
+  for (int i = 0; i < N; ++i) {
+    double r = live ? (double)S[t.rew + lane * N + i] : 0.0;
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) r += __shfl_xor_sync(FULL, r, off);
+    if (lane == 0) red_add(row + i, r);
+    all_done = all_done && done[i] == 1;
+  }
+  if (__any_sync(FULL, all_done)) {
+    const float* info = p.out.info + (size_t)(env0 + (live ? lane : 0)) * N * INFO_F;
+#pragma unroll 1
+    for (int q = 0; q < N * INFO_F; ++q) {
+      double v = all_done ? (double)info[q] : 0.0;
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(FULL, v, off);
+      if (lane == 0) red_add(row + N + q, v);
+    }
+  }
+  const unsigned term = __ballot_sync(FULL, all_done);
+  if (lane == 0) { red_add(row + 15 * N, (double)__popc(term)); red_add(row + 15 * N + 1, (double)nenv); }
+}
+
 constexpr int FORM_WARPS = 1;          // no block-level cooperation: one warp per CTA packs the SM's shared memory best
 #ifndef FM_FORM_MIN_BLOCKS
 #define FM_FORM_MIN_BLOCKS 1           // A/B knob (FM_NVCC_EXTRA=-DFM_FORM_MIN_BLOCKS=n): resident warps ptxas must leave room for
@@ -160,6 +199,7 @@ __global__ void __launch_bounds__(FORM_WARPS * 32, FM_FORM_MIN_BLOCKS) formation
     if (MODE == 0) form_step_env<N, OT>(p, env0 + lane, o); else form_reset_env<N>(p, env0 + lane, o);
   }
   __syncwarp();
+  if (MODE == 0 && p.stats) form_stats<N>(p, S, t, env0, nenv, lane);
   form_emit<N>(p, S, t, env0, nenv, lane, MODE == 0);
 }
 
@@ -199,6 +239,7 @@ __global__ void __launch_bounds__(32, FM_FORM_LOGIC_BLOCKS) formation_logic_kern
     form_step_env<N, OT>(p, env0 + lane, o);
   }
   __syncwarp();
+  if (p.stats) form_stats<N>(p, S, t, env0, nenv, lane);
   float* g_obs = p.out.obs ? p.out.obs + (size_t)env0 * N * F_OBS : nullptr;
   float* g_rew = p.out.reward ? p.out.reward + (size_t)env0 * N : nullptr;
   uint8_t* g_done = p.out.done ? p.out.done + (size_t)env0 * N : nullptr;

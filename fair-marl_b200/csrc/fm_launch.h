@@ -80,6 +80,7 @@ struct FormParams {
   float* pend;               // pending-reset blocks of the split step path ([form_pending_floats][Bp], fm_form.cuh); null: none
   int Bp;                    // B rounded up to whole warps
   int* ready;                // split step path: one flag per 16 envs, logic kernel -> image kernel (programmatic dependent launch); null: none
+  double* stats;             // episode statistics, [ceil(B / 32)][15 N + 2] per-warp partial sums (fm_stats_read layout); null: off
 };
 size_t formation_recipe_floats(int N, int O, int B);
 cudaError_t launch_formation_image(const FormParams& p, cudaStream_t st);   // fm_form_image.cu: node_obs / adj from p.rec

@@ -22,6 +22,11 @@ from fair_marl_b200 import _lib
 from fair_marl_b200.spaces import Box, Discrete
 
 
+# scenario file -> (assignment, fairness_reward): the four formation scenarios this path covers
+SCENARIO_MODES = {"nav_fairassign_fairrew_formation_graph": ("fair", True), "nav_fairassign_nofairrew_formation_graph": ("fair", False),
+                  "nav_base_formation_graph_mask": ("optimal", False), "nav_base_formation_graph_randomgoal": ("random", False)}
+
+
 @dataclass
 class FormationSimConfig:
     """The argparse fields the formation ``Scenario.make_world`` reads (:48-216) that this path honours."""
@@ -51,11 +56,9 @@ class FormationSimConfig:
     def from_args(cls, args: Any, **overrides) -> "FormationSimConfig":
         kw = {f: getattr(args, f) for f in cls.__dataclass_fields__ if hasattr(args, f)}
         name = getattr(args, "scenario_name", "nav_fairassign_fairrew_formation_graph")
-        modes = {"nav_fairassign_fairrew_formation_graph": ("fair", True), "nav_fairassign_nofairrew_formation_graph": ("fair", False),
-                 "nav_base_formation_graph_mask": ("optimal", False), "nav_base_formation_graph_randomgoal": ("random", False)}
-        if name not in modes:
+        if name not in SCENARIO_MODES:
             raise NotImplementedError(f"scenario {name!r} is not one of the four formation scenarios this path covers")
-        kw["assignment"], kw["fairness_reward"] = modes[name]
+        kw["assignment"], kw["fairness_reward"] = SCENARIO_MODES[name]
         for unsupported in ("num_scripted_agents",):
             if getattr(args, unsupported, 0):
                 raise NotImplementedError(f"{unsupported} > 0 is not supported by the formation kernels")
@@ -109,12 +112,14 @@ def share_vec_env_tuple(out: Dict[str, np.ndarray], with_min_time: bool = True):
 
 class B200FormationVecEnv:
     """B formation envs on one GPU.  ``reset_tensor()`` / ``step_tensor(actions int32 [B,N])`` return dicts of CUDA
-    tensors (views of buffers owned by this object, overwritten by the next call)."""
+    tensors (views of buffers owned by this object, overwritten by the next call), or of the caller's arrays with
+    ``out=`` (e.g. the slabs of a ``DeviceRolloutBuffer``).  ``episode_stats``: the steps add up, on the device, the
+    statistics vector of ``read_stats`` (off by default: it costs the step kernels a little)."""
 
     closed = False
 
     def __init__(self, cfg: FormationSimConfig, num_envs: int, device: int = 0, seed: int = 0, env_offset: int = 0,
-                 num_slots: int = 1):
+                 num_slots: int = 1, episode_stats: bool = False):
         torch = _lib.require_cuda()
         self.torch, self.lib, self.cfg = torch, _lib.load(), cfg
         self.num_envs, self.num_agents, self.num_entities = int(num_envs), cfg.num_agents, cfg.num_entities
@@ -153,34 +158,79 @@ class B200FormationVecEnv:
         self.agent_id_observation_space = [Box(-inf, inf, (1,)) for _ in range(N)]
         self.share_agent_id_observation_space = [Box(-inf, inf, (N,)) for _ in range(N)]
         self._out = self._outs[0]
+        if episode_stats:
+            _lib.check(self.lib.fm_formation_stats_enable(self._h, 1, self._stream()), "fm_formation_stats_enable")
 
     def _stream(self):
         return C.c_void_p(self.torch.cuda.current_stream(self.device).cuda_stream)
 
-    def reset_tensor(self, mask=None) -> Dict[str, Any]:
+    def _check_out(self, out: Dict[str, Any], with_step: bool) -> Dict[str, Any]:
+        """Caller-owned output arrays: contiguous CUDA tensors of the API shapes on this env's device, ``adj`` one matrix
+        per env ``[B,E,E]``.  Returns them under the keys of the result dicts, with the env's own info rows."""
+        t, B, N, E = self.torch, self.num_envs, self.num_agents, self.num_entities
+        want = {"obs": ((B, N, _lib.FORMATION_OBS_DIM), t.float32), "node_obs": ((B, N, E, _lib.FORMATION_NODE_FEAT_DIM), t.float32),
+                "adj": ((B, E, E), t.float32)}
+        if with_step:
+            want.update(reward=((B, N), t.float32), done=((B, N), t.uint8))
+        views = {}
+        for name, (shape, dt) in want.items():
+            x = out.get(name)
+            if x is None or tuple(x.shape) != shape or x.dtype != dt or not x.is_contiguous() or x.device != self.device:
+                raise ValueError(f"out[{name!r}] must be a contiguous {dt} tensor of shape {shape} on {self.device}")
+            views["adj_env" if name == "adj" else name] = x
+        if with_step:
+            views["info"] = self._slots[0]["info"]
+        return views
+
+    @staticmethod
+    def _outputs(views: Dict[str, Any]) -> _lib.FmOutputs:
+        return _lib.FmOutputs(*[views[k].data_ptr() if k in views else None
+                                for k in ("obs", "node_obs", "adj_env", "reward", "done", "info")])
+
+    def reset_tensor(self, mask=None, out: Optional[Dict[str, Any]] = None) -> Dict[str, Any]:
+        """Reset all envs (or those with ``mask`` != 0, [B]); returns ``obs``, ``node_obs``, ``adj_env``.  ``out``: write
+        into the caller's ``obs [B,N,11]``, ``node_obs [B,N,E,13]``, ``adj [B,E,E]`` instead of the env's buffers."""
         t = self.torch
+        views = self._check_out(out, with_step=False) if out is not None else None
         m = None
         if mask is not None:
             m = t.as_tensor(np.asarray(mask) if not t.is_tensor(mask) else mask).to(device=self.device, dtype=t.uint8).contiguous()
             if tuple(m.shape) != (self.num_envs,):
                 raise ValueError(f"mask must have shape ({self.num_envs},)")
-        _lib.check(self.lib.fm_formation_reset(self._h, m.data_ptr() if m is not None else None, C.byref(self._out),
+        o = self._outputs(views) if views is not None else self._out
+        _lib.check(self.lib.fm_formation_reset(self._h, m.data_ptr() if m is not None else None, C.byref(o),
                                                self._stream()), "fm_formation_reset")
         if m is not None:
             t.cuda.current_stream(self.device).synchronize()          # keep `m` alive until consumed
-        return {k: self._buf[k] for k in ("obs", "node_obs", "adj_env")}
+        return dict(views) if views is not None else {k: self._buf[k] for k in ("obs", "node_obs", "adj_env")}
 
-    def step_tensor(self, actions) -> Dict[str, Any]:
+    def step_tensor(self, actions, out: Optional[Dict[str, Any]] = None) -> Dict[str, Any]:
+        """One step; ``actions`` int32 CUDA ``[B,N]``.  ``out``: write into the caller's ``obs``, ``node_obs``,
+        ``adj [B,E,E]``, ``reward [B,N]`` float32 and ``done [B,N]`` uint8 (the slabs ``DeviceRolloutBuffer.env_views``
+        hands out) instead of the next slot of the ring, which then does not advance.  Same keys either way."""
         t = self.torch
         if not (t.is_tensor(actions) and actions.is_cuda and actions.dtype == t.int32 and actions.is_contiguous()
                 and tuple(actions.shape) == (self.num_envs, self.num_agents)):
             raise ValueError(f"actions must be a contiguous int32 CUDA tensor [{self.num_envs},{self.num_agents}]")
-        self._slot = (self._slot + 1) % len(self._slots)
-        self._buf, self._out = self._slots[self._slot], self._outs[self._slot]
-        _lib.check(self.lib.fm_formation_step(self._h, actions.data_ptr(), C.byref(self._out), self._stream()),
+        if out is not None:
+            res = self._check_out(out, with_step=True)
+            o = self._outputs(res)
+        else:
+            self._slot = (self._slot + 1) % len(self._slots)
+            self._buf, self._out = self._slots[self._slot], self._outs[self._slot]
+            res, o = dict(self._buf), self._out
+        _lib.check(self.lib.fm_formation_step(self._h, actions.data_ptr(), C.byref(o), self._stream()),
                    "fm_formation_step")
-        out = dict(self._buf)
-        out["done"] = self._buf["done"].view(t.bool)
+        res["done"] = res["done"].view(t.bool)
+        return res
+
+    def read_stats(self, clear: bool = False, out=None):
+        """Local episode-statistics vector (float64 CUDA tensor [15N+2], the layout of ``fm_stats_read``; see
+        ``sharding.stats_layout`` / ``EpisodeStats``).  Needs ``episode_stats=True``.  ``out``: reuse a tensor."""
+        t = self.torch
+        if out is None:
+            out = t.empty(self.lib.fm_stats_len(self.num_agents), dtype=t.float64, device=self.device)
+        _lib.check(self.lib.fm_formation_stats_read(self._h, out.data_ptr(), int(clear), self._stream()), "fm_formation_stats_read")
         return out
 
     def rollout_tensor(self, actions):

@@ -125,7 +125,8 @@ class DeviceRolloutBuffer:
 
 class RolloutCollector:
     """The step loop of ``GMPERunner.run`` (graph_mpe_runner.py:60-80) with everything on the device:
-    ``collect`` (policy forward on slab t) -> simulator step writing slab t + 1 -> ``insert``.
+    ``collect`` (policy forward on slab t) -> simulator step writing slab t + 1 -> ``insert``.  ``env`` is a
+    ``B200GraphVecEnv`` or a ``B200FormationVecEnv``; the actor's ``obs_dim`` / ``node_feat_dim`` must be what it emits.
 
     ``max_graphs`` bounds the number of graphs per policy forward (the dense EmbedConv materialises
     ``[graphs, E, E, hidden]`` activations)."""
@@ -135,6 +136,10 @@ class RolloutCollector:
                  **buffer_kw):
         self.env, self.actor, self.critic = env, actor, critic
         cfg = actor.cfg
+        emits = (env.observation_space[0].shape[0], env.node_observation_space[0].shape[-1])
+        if (cfg.obs_dim, cfg.node_feat_dim) != emits:
+            raise ValueError(f"RolloutCollector: the actor takes obs_dim {cfg.obs_dim} / node_feat_dim {cfg.node_feat_dim}, the env "
+                             f"emits {emits[0]} / {emits[1]} (e.g. PolicyConfig(obs_dim=11, node_feat_dim=13) for the formation family)")
         if buffer is None:
             buffer = DeviceRolloutBuffer(env.cfg.episode_length, env.num_envs, env.num_agents, env.num_entities,
                                          obs_dim=cfg.obs_dim, node_feat_dim=cfg.node_feat_dim, hidden_size=cfg.hidden_size,

@@ -583,11 +583,16 @@ class B200GraphVecEnv:
             pass
 
 
-def make_train_env(all_args, device: int = 0, rank: int = 0, world_size: int = 1) -> B200GraphVecEnv:
+def make_train_env(all_args, device: int = 0, rank: int = 0, world_size: int = 1):
     """Drop-in for ``make_train_env`` in onpolicy/scripts/train_mpe.py:21-43 when
-    ``env_name == 'GraphMPE'``: ``n_rollout_threads`` envs, sharded over ranks if world_size > 1."""
+    ``env_name == 'GraphMPE'``: ``n_rollout_threads`` envs, sharded over ranks if world_size > 1.  The four formation
+    scenarios (``formation.SCENARIO_MODES``) give a ``B200FormationVecEnv`` with its episode statistics on."""
+    from fair_marl_b200.formation import SCENARIO_MODES, B200FormationVecEnv, FormationSimConfig
     from fair_marl_b200.sharding import shard_range
     if getattr(all_args, "env_name", "GraphMPE") != "GraphMPE":
         raise NotImplementedError(f"Can not support the {all_args.env_name} environment")
     off, cnt = shard_range(all_args.n_rollout_threads, world_size, rank)
+    if getattr(all_args, "scenario_name", None) in SCENARIO_MODES:
+        return B200FormationVecEnv(FormationSimConfig.from_args(all_args), num_envs=cnt, device=device, seed=all_args.seed,
+                                   env_offset=off, episode_stats=True)
     return B200GraphVecEnv(all_args, num_envs=cnt, device=device, seed=all_args.seed, env_offset=off)

@@ -218,7 +218,8 @@ int fm_edge_list(int device, const float* adj, int32_t num_graphs, int32_t E, do
  *   [N .. N + 14 N)     per agent, the 14 info values summed over envs at their terminal step
  *   [15 N]              finished episodes,   [15 N + 1]  env-steps
  * fm_stats_read reduces the per-warp partial sums in a fixed order (deterministic) into
- * out_dev (device, K doubles); the caller all-reduces it across ranks (NCCL sum). */
+ * out_dev (device, K doubles); the caller all-reduces it across ranks (NCCL sum).  The formation family has the same
+ * vector through fm_formation_stats_enable / fm_formation_stats_read (below). */
 int fm_stats_len(int32_t num_agents);
 int fm_stats_read(FmHandle* h, double* out_dev, int32_t clear, void* stream);
 
@@ -302,6 +303,17 @@ int fm_formation_step(FmFormation* h, const int32_t* actions, const FmOutputs* o
 int fm_formation_step_many(FmFormation* h, const int32_t* actions, int32_t T, const FmOutputs* outs, void* stream);
 int fm_formation_set_state(FmFormation* h, const FmFormationState* st, void* stream);
 int fm_formation_get_state(FmFormation* h, const FmFormationState* st, void* stream);
+/* Episode statistics of the formation steps: the vector of fm_stats_read, same layout and meaning (K = fm_stats_len(N)).
+ * Per agent the emitted reward (the team total when collaborative) over all env-steps; per agent the 14 info values over
+ * the envs whose agents are all done on that step (once per episode with auto_reset); the number of such envs; env-steps.
+ * Resets add nothing.  Off by default (the logic kernel is a latency-bound chain at its register cap): enable != 0
+ * allocates and clears the per-warp partial sums on first use and attaches them to the steps that follow; 0 detaches them
+ * (they keep their values).  While on, a step whose caller passes no info array writes the info rows into the handle's
+ * own, so the sums do not depend on which outputs are requested.  fm_formation_stats_read reduces the partial sums in a
+ * fixed order (deterministic) into out_dev (device, K doubles) and zeroes them if `clear`; it fails while statistics are
+ * off. */
+int fm_formation_stats_enable(FmFormation* h, int32_t enable, void* stream);
+int fm_formation_stats_read(FmFormation* h, double* out_dev, int32_t clear, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * Fused graph-network forward of the rollout policy (SURVEY.md section 8f, row N2).
