@@ -577,12 +577,21 @@ __global__ void __launch_bounds__(HEAD_WARPS * 32, 1) head_kernel(const __grid_c
       const float lse = mx + logf(se);
       int act = 0;
       if (a.u) {                                             // inverse CDF of softmax(logits)
+        // The fp32 sum of the probabilities can end a few ulps below 1, and u can reach 1 - 2^-24: a u at or above the
+        // sum takes the last action of positive probability, never one that torch.multinomial could not draw.
         const float u = a.u[m];
         float cdf = 0.f;
-        act = a.A - 1;
+        int last = 0;
         bool set = false;
 #pragma unroll
-        for (int o = 0; o < 8; ++o) if (o < a.A) { cdf += expf(lg[o] - lse); if (!set && u < cdf) { act = o; set = true; } }
+        for (int o = 0; o < 8; ++o)
+          if (o < a.A) {
+            const float p = expf(lg[o] - lse);
+            cdf += p;
+            if (p > 0.f) last = o;
+            if (!set && u < cdf) { act = o; set = true; }
+          }
+        if (!set) act = last;
       } else {                                               // FixedCategorical.mode: first maximum
         float best = -INFINITY;
 #pragma unroll
