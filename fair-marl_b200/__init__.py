@@ -6,6 +6,7 @@ missing.  Public surface mirrors the reference interfaces this package replaces:
 
 * ``B200GraphVecEnv``  -- ``onpolicy/envs/env_wrappers.py`` ``GraphSubprocVecEnv`` (ShareVecEnv API)
 * ``solve_fair_assignment`` / ``lexifair_batched`` -- ``marl_fair_assign.py``
+* ``linear_sum_assignment`` / ``min_sum_batched`` -- ``scipy.optimize.linear_sum_assignment`` (square, minimise)
 * ``process_adj`` -- ``onpolicy/algorithms/utils/gnn_new.py:381-413``
 * ``DeviceRolloutBuffer`` / ``RolloutCollector`` -- ``onpolicy/utils/graph_buffer.py`` ``GraphReplayBuffer`` and the
   collect / insert loop of ``onpolicy/runner/shared/graph_mpe_runner.py`` (device-resident, written by the step kernel)
@@ -17,7 +18,8 @@ from fair_marl_b200.build import build_library, library_path            # noqa: 
 from fair_marl_b200.config import SimConfig                             # noqa: F401
 from fair_marl_b200.spaces import Box, Discrete                         # noqa: F401
 from fair_marl_b200.vec_env import B200GraphVecEnv, make_train_env      # noqa: F401
-from fair_marl_b200.assign import lexifair_batched, pair_dist, solve_fair_assignment  # noqa: F401
+from fair_marl_b200.assign import (lexifair_batched, linear_sum_assignment, min_sum_batched, pair_dist,  # noqa: F401
+                                    solve_fair_assignment)
 from fair_marl_b200.edges import process_adj                            # noqa: F401
 from fair_marl_b200.sharding import shard_range, EpisodeStats           # noqa: F401
 from fair_marl_b200.policy import DenseGraphActor, DenseGraphCritic, PolicyConfig, load_reference_state_dict  # noqa: F401
@@ -25,6 +27,6 @@ from fair_marl_b200.rollout import DeviceRolloutBuffer, RolloutCollector  # noqa
 from fair_marl_b200.formation import B200FormationVecEnv, FormationSimConfig  # noqa: F401
 
 __all__ = ["B200GraphVecEnv", "make_train_env", "SimConfig", "Box", "Discrete", "solve_fair_assignment",
-           "lexifair_batched", "pair_dist", "process_adj", "shard_range", "EpisodeStats", "build_library", "library_path",
+           "lexifair_batched", "min_sum_batched", "linear_sum_assignment", "pair_dist", "process_adj", "shard_range", "EpisodeStats", "build_library", "library_path",
            "DenseGraphActor", "DenseGraphCritic", "PolicyConfig", "load_reference_state_dict", "DeviceRolloutBuffer",
            "RolloutCollector", "B200FormationVecEnv", "FormationSimConfig"]

@@ -129,6 +129,8 @@ def load():
         "fm_get_state": ([vp, C.POINTER(FmState), vp], C.c_int),
         "fm_assign_costs": ([C.c_int, vp, i32, i32, vp, vp], C.c_int),
         "fm_assign_positions": ([C.c_int, vp, vp, i32, i32, vp, vp], C.c_int),
+        "fm_assign_min_sum_costs": ([C.c_int, vp, i32, i32, vp, vp], C.c_int),
+        "fm_assign_min_sum_positions": ([C.c_int, vp, vp, i32, i32, vp, vp], C.c_int),
         "fm_pair_dist": ([C.c_int, vp, vp, i64, vp, vp], C.c_int),
         "fm_edge_list": ([C.c_int, vp, i32, i32, C.c_double, i32, i32, i64, vp, vp, vp, vp, vp], C.c_int),
         "fm_stats_read": ([vp, vp, i32, vp], C.c_int),
@@ -161,7 +163,7 @@ def load():
 EXPORTED_SYMBOLS = (
     "fm_abi_version", "fm_last_error", "fm_stats_len", "fm_create", "fm_destroy", "fm_reset", "fm_observe", "fm_soa_stride", "fm_observe_soa", "fm_check_finite", "fm_step",
     "fm_step_onehot", "fm_step_many", "fm_step_host", "fm_step_host_lane", "fm_host_lane_range", "fm_reset_host", "fm_read_info_host", "fm_set_state", "fm_get_state",
-    "fm_assign_costs", "fm_assign_positions", "fm_pair_dist", "fm_edge_list", "fm_stats_read", "fm_num_entities", "fm_mapping",
+    "fm_assign_costs", "fm_assign_positions", "fm_assign_min_sum_costs", "fm_assign_min_sum_positions", "fm_pair_dist", "fm_edge_list", "fm_stats_read", "fm_num_entities", "fm_mapping",
     "fm_algorithmic_bytes_per_step", "fm_kernel_launches",
     "fm_formation_create", "fm_formation_destroy", "fm_formation_reset", "fm_formation_step", "fm_formation_step_many",
     "fm_formation_set_state",

@@ -1,5 +1,6 @@
-"""Batched lexifair goal assignment on the GPU: drop-in for ``marl_fair_assign.solve_fair_assignment``
-(marl_fair_assign.py:16-55; call site navigation_graph.py:555-561)."""
+"""Batched goal assignment on the GPU: lexifair, drop-in for ``marl_fair_assign.solve_fair_assignment``
+(marl_fair_assign.py:16-55; call site navigation_graph.py:555-561), and min-sum, drop-in for
+``scipy.optimize.linear_sum_assignment`` on square matrices (nav_base_formation_graph_mask.py:255-260)."""
 from __future__ import annotations
 
 import numpy as np
@@ -7,13 +8,7 @@ import numpy as np
 from fair_marl_b200 import _lib
 
 
-def lexifair_batched(costs=None, agent_pos=None, goal_pos=None, device: int = 0):
-    """Goal index per agent for a batch of problems, computed on the GPU.
-
-    Either ``costs`` [num, n, n] (float64; torch CUDA tensor or numpy) or ``agent_pos`` / ``goal_pos``
-    [num, n, 2] float32 (costs = float64 Euclidean distances, ``cdist``).  Returns an int32 torch CUDA
-    tensor [num, n] when given tensors, a numpy array when given numpy.
-    """
+def _batched(entry_costs: str, entry_positions: str, costs, agent_pos, goal_pos, device: int):
     torch = _lib.require_cuda()
     lib = _lib.load()
     dev = torch.device("cuda", device)
@@ -26,7 +21,7 @@ def lexifair_batched(costs=None, agent_pos=None, goal_pos=None, device: int = 0)
                 raise ValueError(f"costs must be [num, n, n], got {tuple(c.shape)}")
             num, n = int(c.shape[0]), int(c.shape[1])
             out = torch.empty((num, n), dtype=torch.int32, device=dev)
-            _lib.check(lib.fm_assign_costs(device, c.data_ptr(), num, n, out.data_ptr(), stream), "fm_assign_costs")
+            _lib.check(getattr(lib, entry_costs)(device, c.data_ptr(), num, n, out.data_ptr(), stream), entry_costs)
         else:
             a = torch.as_tensor(agent_pos, dtype=torch.float32, device=dev).contiguous()
             g = torch.as_tensor(goal_pos, dtype=torch.float32, device=dev).contiguous()
@@ -34,9 +29,45 @@ def lexifair_batched(costs=None, agent_pos=None, goal_pos=None, device: int = 0)
                 raise ValueError("agent_pos / goal_pos must both be [num, n, 2]")
             num, n = int(a.shape[0]), int(a.shape[1])
             out = torch.empty((num, n), dtype=torch.int32, device=dev)
-            _lib.check(lib.fm_assign_positions(device, a.data_ptr(), g.data_ptr(), num, n, out.data_ptr(), stream),
-                       "fm_assign_positions")
+            _lib.check(getattr(lib, entry_positions)(device, a.data_ptr(), g.data_ptr(), num, n, out.data_ptr(), stream),
+                       entry_positions)
     return out.cpu().numpy() if as_numpy else out
+
+
+def lexifair_batched(costs=None, agent_pos=None, goal_pos=None, device: int = 0):
+    """Goal index per agent for a batch of problems, computed on the GPU.
+
+    Either ``costs`` [num, n, n] (float64; torch CUDA tensor or numpy) or ``agent_pos`` / ``goal_pos``
+    [num, n, 2] float32 (costs = float64 Euclidean distances, ``cdist``).  Returns an int32 torch CUDA
+    tensor [num, n] when given tensors, a numpy array when given numpy.
+    """
+    return _batched("fm_assign_costs", "fm_assign_positions", costs, agent_pos, goal_pos, device)
+
+
+def min_sum_batched(costs=None, agent_pos=None, goal_pos=None, device: int = 0):
+    """Min-sum matching per problem for a batch, computed on the GPU: ``out[p]`` equals
+    ``scipy.optimize.linear_sum_assignment(costs[p])[1]`` bit for bit, ties included.
+
+    Inputs and return type as ``lexifair_batched``; n <= 32.  A problem with any NaN or +-inf cost gets -1 in
+    every entry of its row.
+    """
+    return _batched("fm_assign_min_sum_costs", "fm_assign_min_sum_positions", costs, agent_pos, goal_pos, device)
+
+
+def linear_sum_assignment(cost_matrix):
+    """Drop-in for ``scipy.optimize.linear_sum_assignment(cost_matrix)`` on a square matrix (minimise), solved on the
+    GPU: ``(row_ind, col_ind)`` as numpy int64, equal to scipy's.  A non-square matrix raises ``ValueError``; so does
+    a matrix with NaN or +-inf entries."""
+    c = np.asarray(cost_matrix, dtype=np.float64)
+    if c.ndim != 2 or c.shape[0] != c.shape[1]:
+        raise ValueError(f"square cost matrix expected, got shape {c.shape}")
+    n = c.shape[0]
+    if n == 0:
+        return np.zeros(0, np.int64), np.zeros(0, np.int64)
+    col = min_sum_batched(costs=c[None])[0]
+    if (col < 0).any():
+        raise ValueError("cost matrix contains NaN or infinite entries")
+    return np.arange(n, dtype=np.int64), col.astype(np.int64)
 
 
 def solve_fair_assignment(costs):

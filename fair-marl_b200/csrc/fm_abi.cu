@@ -819,6 +819,27 @@ int fm_assign_positions(int device, const float* agent_pos, const float* goal_po
   return FM_OK;
 }
 
+int fm_assign_min_sum_costs(int device, const double* costs, int32_t num, int32_t n, int32_t* out, void* stream) {
+  if (num != 0 && (!costs || !out)) return fail(FM_ERR_INVALID_ARG, "fm_assign_min_sum_costs: null argument");
+  if (n < 1 || n > FM_MAX_AGENTS) return fail(FM_ERR_INVALID_ARG, "fm_assign_min_sum_costs: n must be in 1..%d (got %d)", FM_MAX_AGENTS, n);
+  if (num < 0) return fail(FM_ERR_INVALID_ARG, "fm_assign_min_sum_costs: num < 0");
+  int rc = use_device(device);
+  if (rc) return rc;
+  FM_CUDA(fm::launch_lsap(costs, nullptr, nullptr, num, n, out, (cudaStream_t)stream));
+  return FM_OK;
+}
+
+int fm_assign_min_sum_positions(int device, const float* agent_pos, const float* goal_pos, int32_t num, int32_t n,
+                                int32_t* out, void* stream) {
+  if (num != 0 && (!agent_pos || !goal_pos || !out)) return fail(FM_ERR_INVALID_ARG, "fm_assign_min_sum_positions: null argument");
+  if (n < 1 || n > FM_MAX_AGENTS) return fail(FM_ERR_INVALID_ARG, "fm_assign_min_sum_positions: n must be in 1..%d (got %d)", FM_MAX_AGENTS, n);
+  if (num < 0) return fail(FM_ERR_INVALID_ARG, "fm_assign_min_sum_positions: num < 0");
+  int rc = use_device(device);
+  if (rc) return rc;
+  FM_CUDA(fm::launch_lsap(nullptr, agent_pos, goal_pos, num, n, out, (cudaStream_t)stream));
+  return FM_OK;
+}
+
 int fm_pair_dist(int device, const float* a, const float* b, int64_t num, double* out, void* stream) {
   if (!a || !b || !out) return fail(FM_ERR_INVALID_ARG, "fm_pair_dist: null argument");
   if (num < 0) return fail(FM_ERR_INVALID_ARG, "fm_pair_dist: num < 0");
@@ -937,8 +958,6 @@ int fm_formation_create(const FmFormationConfig* cfg, int device, FmFormation** 
   if (cfg->assignment < 0 || cfg->assignment > 2) return fail(FM_ERR_INVALID_ARG, "fm_formation_create: assignment must be 0 (fair), 1 (optimal) or 2 (random)");
   if (cfg->assignment != 0 && cfg->fairness_reward)
     return fail(FM_ERR_INVALID_ARG, "fm_formation_create: the base formation scenarios (optimal / random assignment) have no fairness term");
-  if (cfg->assignment == 1 && cfg->num_agents > 5)
-    return fail(FM_ERR_UNSUPPORTED, "fm_formation_create: the min-sum matching enumerates permutations (num_agents <= 5, got %d)", cfg->num_agents);
   if (cfg->num_obstacles < 0 || cfg->num_obstacles > FM_FORMATION_MAX_OBSTACLES)
     return fail(FM_ERR_INVALID_ARG, "fm_formation_create: num_obstacles must be in 0..%d (got %d)", FM_FORMATION_MAX_OBSTACLES, cfg->num_obstacles);
   if (cfg->episode_length < 1) return fail(FM_ERR_INVALID_ARG, "fm_formation_create: episode_length must be >= 1");

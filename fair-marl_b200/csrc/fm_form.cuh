@@ -418,7 +418,8 @@ __device__ __forceinline__ void f_assign(FEnv<N>& e) {
 }
 
 // Min-sum matching of the current agent -> goal distances by enumeration (scipy linear_sum_assignment in
-// nav_base_formation_graph_mask.py:255-260 and :686-689): match[i] = goal of agent i, delta[i] its distance.  N <= 5.
+// nav_base_formation_graph_mask.py:255-260 and :686-689): match[i] = goal of agent i, delta[i] its distance.  N <= 5
+// (larger teams: f_min_sum_sap below).
 // Takes a COPY of the cost matrix (not the env: the env must not escape to a function that is not inlined).
 template <int N>
 __device__ __noinline__ void f_min_sum_c(const double* __restrict__ cin, int* __restrict__ match, double* __restrict__ delta) {
@@ -442,13 +443,59 @@ __device__ __noinline__ void f_min_sum_c(const double* __restrict__ cin, int* __
   }
   for (int i = 0; i < N; ++i) { match[i] = best[i]; delta[i] = c[i * N + best[i]]; }
 }
+// Min-sum matching for N >= 6, where N! permutations per step are too many: scipy's shortest augmenting path
+// (rectangular_lsap.cpp after Crouse 2016, square case; oracle/lsap.py states it) with its operation order and tie rule,
+// so that match equals scipy's col_ind bit for bit, ties included.  One thread, local arrays; a COPY of the cost matrix
+// like f_min_sum_c.  The warp-per-problem form of the same loop is lsap_kernel (fm_lsap.cu).
+template <int N>
+__device__ __noinline__ void f_min_sum_sap(const double* __restrict__ cin, int* __restrict__ match, double* __restrict__ delta) {
+  double c[N * N], u[N], v[N], spc[N];
+  int col4row[N], row4col[N], path[N], rem[N];
+  bool sr[N], sc[N];
+  for (int k = 0; k < N * N; ++k) c[k] = cin[k];
+  for (int k = 0; k < N; ++k) { u[k] = 0.0; v[k] = 0.0; col4row[k] = -1; row4col[k] = -1; path[k] = -1; }
+  for (int cur = 0; cur < N; ++cur) {
+    for (int k = 0; k < N; ++k) { rem[k] = N - 1 - k; sr[k] = false; sc[k] = false; spc[k] = INFINITY; }
+    double minv = 0.0;
+    int nrem = N, i = cur, sink = -1;
+    while (sink == -1) {
+      sr[i] = true;
+      int index = 0;                     // always set below: an unassigned column stays in rem, and spc is never NaN
+      double lowest = INFINITY;
+      for (int it = 0; it < nrem; ++it) {
+        const int j = rem[it];
+        const double r = minv + c[i * N + j] - u[i] - v[j];       // adds only (nothing to contract), scipy's order
+        if (r < spc[j]) { path[j] = i; spc[j] = r; }
+        if (spc[j] < lowest || (spc[j] == lowest && row4col[j] == -1)) { lowest = spc[j]; index = it; }
+      }
+      minv = lowest;
+      const int j = rem[index];
+      if (row4col[j] == -1) sink = j; else i = row4col[j];
+      sc[j] = true;
+      rem[index] = rem[--nrem];
+    }
+    u[cur] += minv;
+    for (int r = 0; r < N; ++r)
+      if (sr[r] && r != cur) u[r] += minv - spc[col4row[r]];
+    for (int j = 0; j < N; ++j)
+      if (sc[j]) v[j] -= minv - spc[j];
+    for (int j = sink;;) {                                                 // augment along path[] back to row cur
+      const int r = path[j];
+      row4col[j] = r;
+      const int t = col4row[r]; col4row[r] = j; j = t;
+      if (r == cur) break;
+    }
+  }
+  for (int r = 0; r < N; ++r) { match[r] = col4row[r]; delta[r] = c[r * N + col4row[r]]; }
+}
 template <int N>
 __device__ __forceinline__ void f_min_sum(const FEnv<N>& e, int (&match)[N], double (&delta)[N]) {
   double c[N * N], dl[N];
   int m[N];
   FM_UNROLL_N
   for (int k = 0; k < N * N; ++k) c[k] = e.dal[k];
-  f_min_sum_c<N>(c, m, dl);
+  if constexpr (N >= 6) f_min_sum_sap<N>(c, m, dl);
+  else f_min_sum_c<N>(c, m, dl);
   FM_UNROLL_N
   for (int i = 0; i < N; ++i) { match[i] = m[i]; delta[i] = dl[i]; }
 }

@@ -40,6 +40,8 @@ cudaError_t launch_step(const DevParams& p, cudaStream_t st, bool is_reset);
 cudaError_t launch_prefetch(const DevParams& p, cudaStream_t st);   // next-episode placement + assignment (group mapping)
 cudaError_t launch_assign(const double* costs, const float* apos, const float* gpos, int num, int n, int* out,
                           cudaStream_t st);
+// batched min-sum assignment, scipy linear_sum_assignment bit for bit (fm_lsap.cu): one warp per problem, n <= 32
+cudaError_t launch_lsap(const double* costs, const float* apos, const float* gpos, int num, int n, int* out, cudaStream_t st);
 cudaError_t launch_state_io(const DevParams& p, const HostState& hs, int to_internal, cudaStream_t st);
 cudaError_t launch_state_init(const DevParams& p, cudaStream_t st);
 cudaError_t launch_observe_soa(const DevParams& p, float* obs, float* node, float* adj, cudaStream_t st);   // fm_soa.cu

@@ -194,6 +194,17 @@ int fm_assign_costs(int device, const double* costs, int32_t num, int32_t n, int
 int fm_assign_positions(int device, const float* agent_pos, const float* goal_pos, int32_t num,
                         int32_t n, int32_t* out, void* stream);
 
+/* scipy.optimize.linear_sum_assignment (nav_base_formation_graph_mask.py:255-260), batched, square problems, minimise:
+ * one problem per warp, scipy's shortest augmenting path with its operation order and tie rule.  costs: double
+ * [num, n, n]; out: int32 [num, n], out[p][i] = goal of agent i in problem p, equal to scipy's col_ind bit for bit (ties
+ * included).  n <= 32.  A problem with any NaN or +-inf cost gets -1 in every entry of its row (scipy raises or reports
+ * it infeasible); the other problems of the batch are unaffected.  num == 0 does nothing (the pointers may be NULL). */
+int fm_assign_min_sum_costs(int device, const double* costs, int32_t num, int32_t n, int32_t* out, void* stream);
+/* Same from positions: costs = float64 Euclidean distances of float [num, n, 2] inputs, as fm_assign_positions; a NaN or
+ * +-inf coordinate makes its problem's row -1. */
+int fm_assign_min_sum_positions(int device, const float* agent_pos, const float* goal_pos, int32_t num, int32_t n,
+                                int32_t* out, void* stream);
+
 /* Float64 Euclidean distances of `num` pairs of float [.,2] points, out[k] = ||a[k] - b[k]||: the kernels'
  * distance primitive (np.linalg.norm in World.calculate_distances, core.py:204-228; cdist at
  * navigation_graph.py:555), exposed so that its bit-exactness against numpy can be tested directly. */
@@ -254,7 +265,7 @@ typedef struct FmFormationConfig {
   int32_t auto_reset;      /* graphworker, env_wrappers.py:859-865: reset once ALL agents of an env are done */
   int32_t assignment;      /* which goal an agent is rewarded for: 0 'fair' lexifair re-solved every step (:704-721; FA+FR, FA);
                               1 'optimal' min-sum matching re-solved every step (nav_base_formation_graph_mask.py:666-706; OA),
-                              num_agents <= 5; 2 'random' permutation drawn at reset (nav_base_formation_graph_randomgoal.py:
+                              equal to scipy's linear_sum_assignment; 2 'random' permutation drawn at reset (nav_base_formation_graph_randomgoal.py:
                               258-259; RA).  1 and 2 use the base scenarios' 1.5x goal clearance and need fairness_reward 0. */
   int32_t info_every_step; /* 0: info rows are written on the steps on which every agent of the env is done (what the runner reads) */
   int32_t num_walls;       /* 0..2 (:301-333; core.py:36-55, :407-462): E = 2 N + O + W, wall rows of type 3 (:1323-1334) */

@@ -1,6 +1,7 @@
 """Formation kernel timing (diagnostic; the formation family is not a BASELINE config): agent-steps/s of
 fm_formation_step over B envs with CUDA events, and its algorithmic-bytes fraction of the HBM roofline.
-usage: python tools/bench_formation.py [--envs 65536] [--agents 3] [--obstacles 3] [--steps 300]"""
+usage: python tools/bench_formation.py [--envs 65536] [--agents 3] [--obstacles 3] [--steps 300] [--assignment fair]
+--assignment optimal | random: the base scenarios OA / RA (no fairness term); the default is FA+FR."""
 import argparse
 import json
 import os
@@ -20,10 +21,12 @@ def main():
     ap.add_argument("--obstacles", type=int, default=3)
     ap.add_argument("--steps", type=int, default=300)
     ap.add_argument("--warmup", type=int, default=30)
+    ap.add_argument("--assignment", choices=("fair", "optimal", "random"), default="fair")
     a = ap.parse_args()
     B, N, O = a.envs, a.agents, a.obstacles
     E = 2 * N + O
-    cfg = fm.FormationSimConfig(num_agents=N, num_obstacles=O, goal_rew=30.0, collision_rew=30.0)
+    kw = {} if a.assignment == "fair" else dict(assignment=a.assignment, fairness_reward=False)
+    cfg = fm.FormationSimConfig(num_agents=N, num_obstacles=O, goal_rew=30.0, collision_rew=30.0, **kw)
     env = fm.B200FormationVecEnv(cfg, num_envs=B, seed=0)
     env.reset_tensor()
     g = torch.Generator(device="cuda").manual_seed(1234)
@@ -48,9 +51,10 @@ def main():
     if os.path.isfile(pk):
         peak = float(json.load(open(pk))["hbm_gbs"])
     ach = alg / (ms * 1e-3) / 1e9
+    scenario = {"fair": "fairrew", "optimal": "optimal assignment", "random": "random assignment"}[a.assignment]
     print(json.dumps({"metric": "agent-steps/sec, formation step+obs+reward+per-step assignment", "value": B * N / (ms * 1e-3),
                       "unit": "agent-steps/s", "ms_per_step": ms, "steps": a.steps, "warmup": a.warmup,
-                      "config": {"workload": f"formation (fairrew) {N} agents / {N} goals / {O} obstacles, {B} envs, random actions, "
+                      "config": {"workload": f"formation ({scenario}) {N} agents / {N} goals / {O} obstacles, {B} envs, random actions, "
                                              "episode_length 25 with auto-reset", "l2": f"outputs {outs * B / 1e6:.0f} MB per step"},
                       "roofline": {"bound": "hbm", "achieved": ach, "peak": peak, "unit": "GB/s", "frac": ach / peak,
                                    "kernel": f"fm::formation_step_kernel<{N}> (thread per env, float64)",
