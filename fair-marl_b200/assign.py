@@ -39,7 +39,9 @@ def lexifair_batched(costs=None, agent_pos=None, goal_pos=None, device: int = 0)
 
     Either ``costs`` [num, n, n] (float64; torch CUDA tensor or numpy) or ``agent_pos`` / ``goal_pos``
     [num, n, 2] float32 (costs = float64 Euclidean distances, ``cdist``).  Returns an int32 torch CUDA
-    tensor [num, n] when given tensors, a numpy array when given numpy.
+    tensor [num, n] when given tensors, a numpy array when given numpy.  Entries are ordered by
+    (cost, agent, goal), so tied costs have one answer, the oracle's.  A problem with any NaN or +-inf
+    cost (or coordinate) gets -1 in every entry of its row; ``num == 0`` is allowed.
     """
     return _batched("fm_assign_costs", "fm_assign_positions", costs, agent_pos, goal_pos, device)
 
@@ -73,13 +75,15 @@ def linear_sum_assignment(cost_matrix):
 def solve_fair_assignment(costs):
     """Same signature and return convention as the reference function: ``(x, objs)`` with ``x`` the
     0/1 int assignment matrix and ``objs`` the per-agent costs sorted descending
-    (marl_fair_assign.py:54-55)."""
+    (marl_fair_assign.py:54-55).  A matrix with NaN or +-inf entries raises ``ValueError``."""
     costs = np.asarray(costs, dtype=np.float64)
     assert np.ndim(costs) == 2                      # marl_fair_assign.py:6
     n, nj = costs.shape
     if n != nj:
         raise ValueError("square cost matrix expected (num_agents == num_landmarks)")
     match = lexifair_batched(costs=costs[None])[0]
+    if (match < 0).any():
+        raise ValueError("cost matrix contains NaN or infinite entries")
     x = np.zeros((n, nj), dtype=int)
     x[np.arange(n), match] = 1
     objs = np.sort(np.sum(costs * x, axis=1))[::-1]

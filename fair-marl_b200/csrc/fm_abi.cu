@@ -799,7 +799,7 @@ int fm_get_state(FmHandle* h, const FmState* st, void* stream) {
 }
 
 int fm_assign_costs(int device, const double* costs, int32_t num, int32_t n, int32_t* out, void* stream) {
-  if (!costs || !out) return fail(FM_ERR_INVALID_ARG, "fm_assign_costs: null argument");
+  if (num != 0 && (!costs || !out)) return fail(FM_ERR_INVALID_ARG, "fm_assign_costs: null argument");
   if (n < 1 || n > FM_MAX_AGENTS) return fail(FM_ERR_INVALID_ARG, "fm_assign_costs: n must be in 1..%d (got %d)", FM_MAX_AGENTS, n);
   if (num < 0) return fail(FM_ERR_INVALID_ARG, "fm_assign_costs: num < 0");
   int rc = use_device(device);
@@ -810,7 +810,7 @@ int fm_assign_costs(int device, const double* costs, int32_t num, int32_t n, int
 
 int fm_assign_positions(int device, const float* agent_pos, const float* goal_pos, int32_t num, int32_t n,
                         int32_t* out, void* stream) {
-  if (!agent_pos || !goal_pos || !out) return fail(FM_ERR_INVALID_ARG, "fm_assign_positions: null argument");
+  if (num != 0 && (!agent_pos || !goal_pos || !out)) return fail(FM_ERR_INVALID_ARG, "fm_assign_positions: null argument");
   if (n < 1 || n > FM_MAX_AGENTS) return fail(FM_ERR_INVALID_ARG, "fm_assign_positions: n must be in 1..%d (got %d)", FM_MAX_AGENTS, n);
   if (num < 0) return fail(FM_ERR_INVALID_ARG, "fm_assign_positions: num < 0");
   int rc = use_device(device);

@@ -440,7 +440,10 @@ __global__ void __launch_bounds__(THREADS) prefetch_kernel(const __grid_constant
 }
 
 // =============================================================================================
-// Stand-alone batched lexifair (marl_fair_assign.py:16-55).
+// Stand-alone batched lexifair (marl_fair_assign.py:16-55).  A NaN or +-inf cost (or coordinate: dist64 alone would turn a
+// NaN into a distance of 0) breaks the total order the sort relies on, so such a problem gets -1 in every entry of its row
+// instead of an arbitrary permutation; the other problems of the batch are unaffected.  The check lives here, not in
+// lexifair_group, whose other callers (resets, prefetch) solve distances of finite positions.
 template <int G>
 __global__ void __launch_bounds__(THREADS) assign_kernel(const double* __restrict__ costs, const float* __restrict__ apos,
                                                          const float* __restrict__ gpos, int num, int n, int* __restrict__ out) {
@@ -458,15 +461,25 @@ __global__ void __launch_bounds__(THREADS) assign_kernel(const double* __restric
   uint16_t* ord = reinterpret_cast<uint16_t*>(base + 2 * n * n);
   int* asg = reinterpret_cast<int*>(base + 2 * n * n + ((n * n + 1) >> 1));
   if (prob >= num) return;                                        // group-uniform; only group syncs below
+  bool finite = true;
   if (i < n) {
     for (int j = 0; j < n; ++j) {
-      if (costs) cost[i * n + j] = costs[((size_t)prob * n + i) * n + j];
-      else {
-        const float* a = apos + ((size_t)prob * n + i) * 2;
+      if (costs) {
+        const double c = costs[((size_t)prob * n + i) * n + j];
+        finite = finite && isfinite(c);
+        cost[i * n + j] = c;
+      } else {                                                    // dist64 in two halves: a NaN coordinate stays NaN in
+        const float* a = apos + ((size_t)prob * n + i) * 2;       // the square, its root would make it 0
         const float* g = gpos + ((size_t)prob * n + j) * 2;
-        cost[i * n + j] = dist64(a[0], a[1], g[0], g[1]);
+        const double q = dist64_sq(a[0], a[1], g[0], g[1]);
+        finite = finite && isfinite(q);
+        cost[i * n + j] = dsqrt_fast(q);
       }
     }
+  }
+  if (!__all_sync(gmask, finite)) {
+    if (i < n) out[(size_t)prob * n + i] = -1;
+    return;
   }
   __syncwarp(gmask);
   const int g = lexifair_group<G>(cost, ord, asg, n, i, gmask);

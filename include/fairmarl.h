@@ -187,10 +187,13 @@ int fm_get_state(FmHandle* h, const FmState* st, void* stream);
 
 /* marl_fair_assign.solve_fair_assignment (marl_fair_assign.py:16-55), batched: one problem per
  * lane group.  costs: double [num, n, n] (cost[i][j] = agent i -> goal j); out: int32 [num, n]
- * goal index per agent (np.where(x == 1)[1], navigation_graph.py:558).  n <= 32. */
+ * goal index per agent (np.where(x == 1)[1], navigation_graph.py:558).  n <= 32.  Entries are
+ * totally ordered by (cost, i, j), so tied costs have exactly one answer (oracle/lexifair.py).  A
+ * problem with any NaN or +-inf cost gets -1 in every entry of its row; the other problems of the
+ * batch are unaffected.  num == 0 does nothing (the pointers may be NULL). */
 int fm_assign_costs(int device, const double* costs, int32_t num, int32_t n, int32_t* out, void* stream);
 /* Same from positions: cdist(agent_pos, goal_pos) (navigation_graph.py:555) in float64 from
- * float [num, n, 2] inputs. */
+ * float [num, n, 2] inputs; a NaN or +-inf coordinate makes its problem's row -1. */
 int fm_assign_positions(int device, const float* agent_pos, const float* goal_pos, int32_t num,
                         int32_t n, int32_t* out, void* stream);
 
