@@ -79,7 +79,7 @@ class FmFormationState(C.Structure):
 class FmGnnConfig(C.Structure):
     _fields_ = [("num_graphs", C.c_int32), ("graphs_per_adj", C.c_int32), ("num_entities", C.c_int32),
                 ("node_feat_dim", C.c_int32), ("embed_layers", C.c_int32), ("conv_layers", C.c_int32), ("aggr", C.c_int32),
-                ("relu", C.c_int32), ("layer_norm", C.c_int32), ("reserved_", C.c_int32), ("max_edge_dist", C.c_double)]
+                ("relu", C.c_int32), ("layer_norm", C.c_int32), ("mapping", C.c_int32), ("max_edge_dist", C.c_double)]
 
 
 class FmHeadConfig(C.Structure):
@@ -149,6 +149,7 @@ def load():
         "fm_formation_stats_read": ([vp, vp, i32, vp], C.c_int),
         "fm_gnn_weight_floats": ([C.POINTER(FmGnnConfig)], i64),
         "fm_gnn_supported": ([i32, i32], C.c_int),
+        "fm_gnn_mapping": ([i32, i32], C.c_int),
         "fm_gnn_forward": ([C.c_int, C.POINTER(FmGnnConfig), vp, vp, vp, vp, vp, vp], C.c_int),
         "fm_head_weight_floats": ([C.POINTER(FmHeadConfig)], i64),
         "fm_policy_head": ([C.c_int, C.POINTER(FmHeadConfig), vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp], C.c_int),
@@ -167,7 +168,8 @@ EXPORTED_SYMBOLS = (
     "fm_algorithmic_bytes_per_step", "fm_kernel_launches",
     "fm_formation_create", "fm_formation_destroy", "fm_formation_reset", "fm_formation_step", "fm_formation_step_many",
     "fm_formation_set_state",
-    "fm_formation_get_state", "fm_formation_stats_enable", "fm_formation_stats_read", "fm_gnn_weight_floats", "fm_gnn_supported", "fm_gnn_forward",
+    "fm_formation_get_state", "fm_formation_stats_enable", "fm_formation_stats_read", "fm_gnn_weight_floats", "fm_gnn_supported", "fm_gnn_mapping",
+    "fm_gnn_forward",
     "fm_head_weight_floats", "fm_policy_head",
 )
 

@@ -1179,12 +1179,24 @@ int fm_gnn_supported(int32_t num_entities, int32_t node_feat_dim) {
   return fm::gnn_supported_entities(num_entities) && node_feat_dim >= 2 && node_feat_dim <= 17 ? 1 : 0;
 }
 
+int fm_gnn_mapping(int32_t num_entities, int32_t node_feat_dim) {
+  if (node_feat_dim < 2 || node_feat_dim > 17) return 0;
+  if (fm::gnn_supported_entities(num_entities)) return 1;
+  return fm::gnn_wide_supported_entities(num_entities) ? 2 : 0;
+}
+
 int fm_gnn_forward(int device, const FmGnnConfig* cfg, const float* weights, const float* node_obs, const float* adj,
                    const int32_t* agent_id, float* out, void* stream) {
   if (!cfg || !weights || !node_obs || !adj || !out) return fail(FM_ERR_INVALID_ARG, "fm_gnn_forward: null argument");
   if (cfg->num_graphs < 0 || cfg->graphs_per_adj < 1) return fail(FM_ERR_INVALID_ARG, "fm_gnn_forward: bad graph counts");
-  if (!fm_gnn_supported(cfg->num_entities, cfg->node_feat_dim))
-    return fail(FM_ERR_UNSUPPORTED, "fm_gnn_forward: not compiled for %d entities x %d features", cfg->num_entities, cfg->node_feat_dim);
+  if (cfg->mapping < 0 || cfg->mapping > 2)
+    return fail(FM_ERR_INVALID_ARG, "fm_gnn_forward: mapping %d (0 auto, 1 warp per graph, 2 CTA per graph)", cfg->mapping);
+  const int E = cfg->num_entities, NF = cfg->node_feat_dim;
+  const bool ok = cfg->mapping == 0 ? fm_gnn_mapping(E, NF) != 0
+                : cfg->mapping == 1 ? fm_gnn_supported(E, NF) != 0
+                                    : fm::gnn_wide_supported_entities(E) && NF >= 2 && NF <= 17;
+  if (!ok)
+    return fail(FM_ERR_UNSUPPORTED, "fm_gnn_forward: mapping %d is not available for %d entities x %d features", cfg->mapping, E, NF);
   if (cfg->embed_layers < 0 || cfg->embed_layers > 2 || cfg->conv_layers < 1 || cfg->conv_layers > 8 || cfg->aggr < 0 || cfg->aggr > 3)
     return fail(FM_ERR_UNSUPPORTED, "fm_gnn_forward: embed_layers %d / conv_layers %d / aggr %d", cfg->embed_layers, cfg->conv_layers, cfg->aggr);
   int rc = use_device(device);

@@ -91,7 +91,9 @@ size_t formation_pending_floats(int N, int O, int B);
 cudaError_t launch_formation_prefetch(const FormParams& p, cudaStream_t st);   // fm_form_image.cu
 cudaError_t launch_formation(const FormParams& p, bool is_reset, cudaStream_t st, const FormAsync* async = nullptr);
 // fused graph-network forward of the rollout policy (fm_policy.cu)
-bool gnn_supported_entities(int E);
+bool gnn_supported_entities(int E);        // warp per graph (gnn_kernel<E, RELU>): compiled for E
+constexpr int GNN_WIDE_MAX_ENTITIES = 2 * FM_MAX_AGENTS;
+bool gnn_wide_supported_entities(int E);   // CTA per graph (gnn_wide_kernel<EMAX, RELU>): 2 <= E <= 64
 int gnn_weight_count(int embed_layers, int conv_layers);
 cudaError_t launch_gnn(const FmGnnConfig& c, const float* weights, const float* node, const float* adj, const int* agent_id,
                        float* out, cudaStream_t st);

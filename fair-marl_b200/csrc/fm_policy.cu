@@ -388,6 +388,320 @@ static cudaError_t gnn_launch_e(const GnnArgs& a, cudaStream_t st) {
   return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Second mapping of the same forward, for any 2 <= E <= 64 known only at run time: one CTA of GW_THREADS threads per graph
+// (persistent over graphs), the weights in shared memory once per CTA, the graph's scratch (the warp kernel's layout,
+// sized by the run-time E) after them.  A warp's scratch at E = 32 would already be 24 KB, so the warp-per-graph layout
+// cannot hold these shapes; here the whole CTA works on one graph and block barriers replace __syncwarp.
+//   thread (t, j), t = tid / P, j = tid % P: target t, sources j, j + P, ...  (P = GW_THREADS / EMAX adjacent lanes of one
+//   warp, so a target's partial sums are still combined with shuffles in lane order);
+//   stage B1: warp w projects nodes w, w + 4, w + 8, ... (lane = 5 output columns, as in the warp kernel);
+//   stage B2 + B3: one head at a time, the target's scores in SPL = EMAX / P registers per thread.
+// Every output element is computed by one thread in a fixed order: deterministic, and the bits of a graph do not depend on
+// the CTA or the round of the persistent loop that computes it.
+constexpr int GW_THREADS = 128;
+
+__host__ __device__ inline int gnn_wide_scratch_floats(int E) {
+  return ((E * E + 3) & ~3) + E * (GnnLayout<1>::NFP + GXS + GQS);
+}
+
+template <int EMAX, bool RELU>
+__global__ void __launch_bounds__(GW_THREADS, 2) gnn_wide_kernel(const __grid_constant__ GnnArgs a, const int E) {
+  constexpr int P = GW_THREADS / EMAX;                        // threads per target
+  constexpr int SPL = EMAX / P;                               // sources per thread (at most)
+  constexpr int NFP = GnnLayout<1>::NFP;
+  constexpr int NB = 8;                                       // B1: nodes per warp and pass
+  constexpr int NW = GW_THREADS / 32;
+  static_assert(P >= 1 && 32 % P == 0 && SPL * P == EMAX, "a target's threads must sit in one warp");
+  extern __shared__ __align__(16) float smem[];
+  float* W = smem;
+  const int wpad = (a.wfloats + 3) & ~3;
+  const int tid = threadIdx.x, lane = tid & 31, wib = tid >> 5;
+  for (int k = tid; k < a.wfloats; k += GW_THREADS) W[k] = __ldg(a.w + k);
+  float* s_adj = smem + wpad;
+  float* s_feat = s_adj + ((E * E + 3) & ~3);
+  float* s_x = s_feat + E * NFP;
+  float* s_q = s_x + E * GXS;
+  const bool ln = a.ln != 0;
+  const int NF = a.NF, KF = NF - 1;
+  const int t = tid / P, j = tid - t * P;
+  const bool tl = t < E;
+  const unsigned tmask = __ballot_sync(FULL, tl);
+  __syncthreads();
+
+  for (int m = blockIdx.x; m < a.M; m += gridDim.x) {
+    // ---- inputs -> scratch ---------------------------------------------------------------------------------
+    {
+      const float* ga = a.adj + (size_t)(m / a.rep) * E * E;
+      for (int k = tid; k < E * E; k += GW_THREADS) s_adj[k] = __ldg(ga + k);
+      const float* gn = a.node + (size_t)m * E * NF;
+      for (int k = tid; k < E * NF; k += GW_THREADS) { const int n = k / NF; s_feat[n * NFP + (k - n * NF)] = __ldcs(gn + k); }
+    }
+    __syncthreads();
+    // ---- A0: hn[n][c] -> s_x -------------------------------------------------------------------------------
+    for (int o = tid; o < E * GH; o += GW_THREADS) {
+      const int n = o >> 4, c = o & 15;
+      const float* f = s_feat + n * NFP;
+      const int ty = min(max((int)f[KF], 0), 3);
+      float acc = W[GW_TYPE + ty * GH + c];
+      for (int k = 0; k < KF; ++k) acc = fmaf(W[GW_WN + k * GH + c], f[k], acc);
+      s_x[n * GXS + c] = acc;
+    }
+    __syncthreads();
+    // ---- A: edge messages, summed at the target -------------------------------------------------------------
+    {
+      // compensated (Kahan) sums: a thread adds up to 32 messages here, where a warp-kernel lane adds at most 19, and the
+      // rounding of a long fp32 chain would otherwise grow with E
+      float acc[GH], cmp[GH];
+#pragma unroll
+      for (int f = 0; f < GH; ++f) { acc[f] = 0.f; cmp[f] = 0.f; }
+      if (tl) {
+#pragma unroll 1
+        for (int r = j; r < E; r += P) {
+          const float d = s_adj[r * E + t];                   // edge r -> t
+          if (!(d < a.max_edge_dist && d > 0.0f)) continue;   // process_adj: strict <, > 0
+          float h[GH];
+#pragma unroll
+          for (int f = 0; f < GH; f += 4) {
+            const float4 hn = *reinterpret_cast<const float4*>(s_x + r * GXS + f);
+            const float4 wd = *reinterpret_cast<const float4*>(W + GW_WD + f);
+            h[f] = g_act<RELU>(fmaf(wd.x, d, hn.x)); h[f + 1] = g_act<RELU>(fmaf(wd.y, d, hn.y));
+            h[f + 2] = g_act<RELU>(fmaf(wd.z, d, hn.z)); h[f + 3] = g_act<RELU>(fmaf(wd.w, d, hn.w));
+          }
+          g_layer_norm(h, W + GW_LN1, ln);
+          for (int l = 0; l < a.embed_layers; ++l) {
+            const float* wl = W + GW_EMBED_END + l * GW_HID;
+            float o[GH];
+#pragma unroll
+            for (int g = 0; g < GH; g += 4) {
+              const float4 b = *reinterpret_cast<const float4*>(wl + GH * GH + g);
+              o[g] = b.x; o[g + 1] = b.y; o[g + 2] = b.z; o[g + 3] = b.w;
+            }
+#pragma unroll
+            for (int f = 0; f < GH; ++f) {
+#pragma unroll
+              for (int g = 0; g < GH; g += 4) {
+                const float4 w4 = *reinterpret_cast<const float4*>(wl + f * GH + g);
+                o[g] = fmaf(w4.x, h[f], o[g]); o[g + 1] = fmaf(w4.y, h[f], o[g + 1]);
+                o[g + 2] = fmaf(w4.z, h[f], o[g + 2]); o[g + 3] = fmaf(w4.w, h[f], o[g + 3]);
+              }
+            }
+#pragma unroll
+            for (int g = 0; g < GH; ++g) h[g] = g_act<RELU>(o[g]);
+            g_layer_norm(h, wl + GH * GH + GH, ln);
+          }
+#pragma unroll
+          for (int f = 0; f < GH; ++f) {
+            const float y = h[f] - cmp[f], t2 = acc[f] + y;
+            cmp[f] = (t2 - acc[f]) - y;
+            acc[f] = t2;
+          }
+        }
+      }
+      // the P partial sums of a target, in lane order
+#pragma unroll
+      for (int f = 0; f < GH; ++f) {
+        float v = acc[f];
+#pragma unroll
+        for (int o = 1; o < P; ++o) { const float u = __shfl_down_sync(FULL, acc[f], o); if (j + o < P) v += u; }
+        acc[f] = v;
+      }
+      __syncthreads();                                        // every thread has read hn before s_x is overwritten
+      if (tl && j == 0) {
+#pragma unroll
+        for (int f = 0; f < GH; f += 4) *reinterpret_cast<float4*>(s_x + t * GXS + f) = make_float4(acc[f], acc[f + 1], acc[f + 2], acc[f + 3]);
+      }
+    }
+    __syncthreads();
+    // ---- convs ----------------------------------------------------------------------------------------------
+    for (int layer = 0; layer < a.conv_layers; ++layer) {
+      const float* wc = W + GW_EMBED_END + a.embed_layers * GW_HID + layer * GW_CONV;
+      const float* bc = wc + GH * GQW;
+      const float* we = bc + GQW;
+      // B1: [q | k | v | skip][n][col] for col = lane + 32 u, u < 5; warp wib takes nodes wib, wib + NW, ...
+      {
+#pragma unroll 1
+        for (int n0 = wib; n0 < E; n0 += NW * NB) {
+          float acc[NB][5];
+#pragma unroll
+          for (int u = 0; u < 5; ++u) {
+            const float b = bc[lane + 32 * u];
+#pragma unroll
+            for (int n = 0; n < NB; ++n) acc[n][u] = b;
+          }
+#pragma unroll
+          for (int k0 = 0; k0 < GH; k0 += 4) {
+            float w[4][5];
+#pragma unroll
+            for (int kk = 0; kk < 4; ++kk)
+#pragma unroll
+              for (int u = 0; u < 5; ++u) w[kk][u] = wc[(k0 + kk) * GQW + lane + 32 * u];
+#pragma unroll
+            for (int n = 0; n < NB; ++n) {
+              if (n0 + n * NW < E) {
+                const float4 x4 = *reinterpret_cast<const float4*>(s_x + (n0 + n * NW) * GXS + k0);
+#pragma unroll
+                for (int u = 0; u < 5; ++u) {
+                  acc[n][u] = fmaf(w[0][u], x4.x, acc[n][u]); acc[n][u] = fmaf(w[1][u], x4.y, acc[n][u]);
+                  acc[n][u] = fmaf(w[2][u], x4.z, acc[n][u]); acc[n][u] = fmaf(w[3][u], x4.w, acc[n][u]);
+                }
+              }
+            }
+          }
+#pragma unroll
+          for (int n = 0; n < NB; ++n)
+            if (n0 + n * NW < E) {
+#pragma unroll
+              for (int u = 0; u < 5; ++u) s_q[(n0 + n * NW) * GQS + lane + 32 * u] = acc[n][u];
+            }
+        }
+      }
+      __syncthreads();                                        // s_q complete; s_x (the layer input) is dead from here
+      // B2 + B3: attention of target t over its sources, one head at a time
+      {
+        float out[GH];
+#pragma unroll
+        for (int c = 0; c < GH; ++c) out[c] = 0.f;
+        float adsum[GHEADS] = {0.f, 0.f, 0.f};
+        if (tl) {
+#pragma unroll
+          for (int h = 0; h < GHEADS; ++h) {
+            float q[GH];
+#pragma unroll
+            for (int c = 0; c < GH; c += 4) {
+              const float4 q4 = *reinterpret_cast<const float4*>(s_q + t * GQS + h * GH + c);
+              q[c] = q4.x; q[c + 1] = q4.y; q[c + 2] = q4.z; q[c + 3] = q4.w;
+            }
+            float qe = 0.f;
+#pragma unroll
+            for (int c = 0; c < GH; ++c) qe = fmaf(q[c], we[h * GH + c], qe);
+            float sc[SPL];
+#pragma unroll
+            for (int i = 0; i < SPL; ++i) {
+              const int s = j + i * P;
+              float v = -INFINITY;
+              if (s < E) {
+                const float d = s_adj[s * E + t];             // edge s -> t
+                if (d < a.max_edge_dist && d > 0.0f) {
+                  float dot = 0.f;
+#pragma unroll
+                  for (int c = 0; c < GH; c += 4) {
+                    const float4 k4 = *reinterpret_cast<const float4*>(s_q + s * GQS + GHC + h * GH + c);
+                    dot = fmaf(q[c], k4.x, dot); dot = fmaf(q[c + 1], k4.y, dot);
+                    dot = fmaf(q[c + 2], k4.z, dot); dot = fmaf(q[c + 3], k4.w, dot);
+                  }
+                  v = (dot + qe * d) * 0.25f;                 // 1 / sqrt(16)
+                }
+              }
+              sc[i] = v;
+            }
+            // softmax over the sources of (h, t): P threads x SPL entries
+            float mx = -INFINITY;
+#pragma unroll
+            for (int i = 0; i < SPL; ++i) mx = fmaxf(mx, sc[i]);
+#pragma unroll
+            for (int o = 1; o < P; ++o) mx = fmaxf(mx, __shfl_sync(tmask, mx, (lane & ~(P - 1)) + ((j + o) % P)));
+            float sum = 0.f;
+#pragma unroll
+            for (int i = 0; i < SPL; ++i) { const float ex = sc[i] == -INFINITY ? 0.f : expf(sc[i] - mx); sc[i] = ex; sum += ex; }
+            float tot = 0.f;                                   // fixed order: thread j = 0, 1, ... of the target
+#pragma unroll
+            for (int o = 0; o < P; ++o) tot += __shfl_sync(tmask, sum, (lane & ~(P - 1)) + o);
+            const float inv = tot > 0.f ? 1.0f / tot : 0.f;   // targets without incoming edges: alpha = 0 (nan_to_num)
+            // weighted values of this head, summed apart from the other heads' (shorter fp32 chains), compensated
+            float ph[GH], pc[GH];
+#pragma unroll
+            for (int c = 0; c < GH; ++c) { ph[c] = 0.f; pc[c] = 0.f; }
+#pragma unroll
+            for (int i = 0; i < SPL; ++i) {
+              const int s = j + i * P;
+              if (s < E) {
+                const float al = sc[i] * inv;
+                adsum[h] = fmaf(al, s_adj[s * E + t], adsum[h]);
+#pragma unroll
+                for (int c = 0; c < GH; c += 4) {
+                  const float4 v4 = *reinterpret_cast<const float4*>(s_q + s * GQS + 2 * GHC + h * GH + c);
+                  const float vv[4] = {v4.x, v4.y, v4.z, v4.w};
+#pragma unroll
+                  for (int q4 = 0; q4 < 4; ++q4) {
+                    const float y = al * vv[q4] - pc[c + q4], t2 = ph[c + q4] + y;
+                    pc[c + q4] = (t2 - ph[c + q4]) - y;
+                    ph[c + q4] = t2;
+                  }
+                }
+              }
+            }
+#pragma unroll
+            for (int c = 0; c < GH; ++c) out[c] += ph[c];
+          }
+        }
+        // combine the P threads of a target (lane order), add the edge term, mean over heads, skip, activation
+#pragma unroll
+        for (int c = 0; c < GH; ++c) {
+          float v = out[c];
+#pragma unroll
+          for (int o = 1; o < P; ++o) { const float u = __shfl_down_sync(FULL, out[c], o); if (j + o < P) v += u; }
+          out[c] = v;
+        }
+#pragma unroll
+        for (int h = 0; h < GHEADS; ++h) {
+          float v = adsum[h];
+#pragma unroll
+          for (int o = 1; o < P; ++o) { const float u = __shfl_down_sync(FULL, adsum[h], o); if (j + o < P) v += u; }
+          adsum[h] = v;
+        }
+        if (tl && j == 0) {
+#pragma unroll
+          for (int c = 0; c < GH; ++c) {
+            float v = out[c];
+#pragma unroll
+            for (int h = 0; h < GHEADS; ++h) v = fmaf(adsum[h], we[h * GH + c], v);
+            v = v * (1.0f / GHEADS) + s_q[t * GQS + 3 * GHC + c];
+            s_x[t * GXS + c] = g_act<RELU>(v);
+          }
+        }
+      }
+      __syncthreads();                                        // s_x complete; s_q free for the next layer
+    }
+    // ---- aggregation ----------------------------------------------------------------------------------------
+    if (tid < GH) {
+      float v;
+      if (a.aggr == 0) {
+        const int node = a.agent_id ? a.agent_id[m] : (m % a.rep);
+        v = s_x[min(max(node, 0), E - 1) * GXS + tid];
+      } else {
+        v = s_x[tid];
+        for (int n = 1; n < E; ++n) { const float u = s_x[n * GXS + tid]; v = a.aggr == 2 ? fmaxf(v, u) : v + u; }
+        if (a.aggr == 1) v *= 1.0f / (float)E;
+      }
+      a.out[(size_t)m * GH + tid] = v;
+    }
+    __syncthreads();                                          // the scratch is read before the next graph overwrites it
+  }
+}
+
+template <int EMAX, bool RELU>
+static cudaError_t gnn_wide_launch_k(const GnnArgs& a, int E, size_t smem, int sms, cudaStream_t st) {
+  cudaError_t e = cudaFuncSetAttribute(gnn_wide_kernel<EMAX, RELU>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  int per_sm = 0;
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gnn_wide_kernel<EMAX, RELU>, GW_THREADS, smem);
+  if (e != cudaSuccess) return e;
+  if (per_sm < 1) return cudaErrorInvalidConfiguration;
+  const int grid = a.M < per_sm * sms ? a.M : per_sm * sms;
+  gnn_wide_kernel<EMAX, RELU><<<grid, GW_THREADS, smem, st>>>(a, E);
+  return cudaGetLastError();
+}
+
+static cudaError_t gnn_wide_launch(const GnnArgs& a, int E, cudaStream_t st) {
+  const size_t smem = (size_t)(((a.wfloats + 3) & ~3) + gnn_wide_scratch_floats(E)) * sizeof(float);
+  int dev = 0, sms = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (e != cudaSuccess) return e;
+  if (E <= 32) return a.relu ? gnn_wide_launch_k<32, true>(a, E, smem, sms, st) : gnn_wide_launch_k<32, false>(a, E, smem, sms, st);
+  return a.relu ? gnn_wide_launch_k<64, true>(a, E, smem, sms, st) : gnn_wide_launch_k<64, false>(a, E, smem, sms, st);
+}
+
 // E values compiled: the navigation / formation shapes at N = 2..7 with O <= 3 and up to 2 walls
 #define FM_GNN_CASES(X) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(17) X(19)
 
@@ -398,6 +712,8 @@ bool gnn_supported_entities(int E) {
   return false;
 }
 
+bool gnn_wide_supported_entities(int E) { return E >= 2 && E <= GNN_WIDE_MAX_ENTITIES; }
+
 cudaError_t launch_gnn(const FmGnnConfig& c, const float* weights, const float* node, const float* adj, const int* agent_id,
                        float* out, cudaStream_t st) {
   GnnArgs a;
@@ -407,6 +723,9 @@ cudaError_t launch_gnn(const FmGnnConfig& c, const float* weights, const float* 
   a.max_edge_dist = (float)c.max_edge_dist;
   a.wfloats = gnn_weight_floats(c.embed_layers, c.conv_layers);
   if (a.M <= 0) return cudaSuccess;
+  const int mapping = c.mapping != 0 ? c.mapping : (gnn_supported_entities(c.num_entities) ? 1 : 2);
+  if (mapping == 2) return gnn_wide_supported_entities(c.num_entities) ? gnn_wide_launch(a, c.num_entities, st) : cudaErrorInvalidValue;
+  if (mapping != 1) return cudaErrorInvalidValue;
 #define X(e) if (c.num_entities == e) return gnn_launch_e<e>(a, st);
   FM_GNN_CASES(X)
 #undef X

@@ -169,12 +169,13 @@ _AGGR_CODE = {"node": 0, "mean": 1, "max": 2, "add": 3}
 
 
 def fused_gnn_supported(cfg: PolicyConfig, num_entities: int, graph_aggr: str) -> bool:
-    """Shape family of the fused CUDA forward (csrc/fm_policy.cu): the configuration of the shipped model_weights."""
+    """Shape family of the fused CUDA forward (csrc/fm_policy.cu): the configuration of the shipped model_weights, at any
+    graph size a fused kernel covers (``fm_gnn_mapping``: 2 <= E <= 64)."""
     from fair_marl_b200 import _lib
     ok = (cfg.embed_hidden_size == 16 and cfg.gnn_hidden_size == 16 and cfg.gnn_num_heads == 3 and not cfg.gnn_concat_heads
           and cfg.embed_layer_N <= 2 and cfg.num_embeddings <= 4 and cfg.embed_use_ReLU == cfg.gnn_use_ReLU
           and (graph_aggr == "node" or cfg.global_aggr_type in ("mean", "max", "add")))
-    return bool(ok and _lib.load().fm_gnn_supported(int(num_entities), int(cfg.node_feat_dim)))
+    return bool(ok and _lib.load().fm_gnn_mapping(int(num_entities), int(cfg.node_feat_dim)) != 0)
 
 
 def pack_gnn_weights(gnn: "DenseGNNBase") -> Tensor:
@@ -241,9 +242,11 @@ class DenseGNNBase(nn.Module):
             self._pack_key, self._pack = key, pack_gnn_weights(self)
         return self._pack
 
-    def forward_fused(self, node_obs: Tensor, adj_env: Tensor, graphs_per_adj: int, agent_id: Optional[Tensor]) -> Tensor:
+    def forward_fused(self, node_obs: Tensor, adj_env: Tensor, graphs_per_adj: int, agent_id: Optional[Tensor],
+                      mapping: int = 0) -> Tensor:
         """One launch of ``fm_gnn_forward``.  node_obs [M, E, F] contiguous fp32; adj_env [M / graphs_per_adj, E, E];
-        agent_id [M] or [M, 1] node indices (aggr 'node')."""
+        agent_id [M] or [M, 1] node indices (aggr 'node').  ``mapping``: 0 auto, 1 the warp-per-graph kernel, 2 the
+        CTA-per-graph kernel (``FmGnnConfig.mapping``)."""
         import ctypes as C
         from fair_marl_b200 import _lib
         cfg = self.cfg
@@ -254,7 +257,7 @@ class DenseGNNBase(nn.Module):
         c = _lib.FmGnnConfig(num_graphs=M, graphs_per_adj=int(graphs_per_adj), num_entities=E, node_feat_dim=F,
                              embed_layers=cfg.embed_layer_N, conv_layers=1 + cfg.gnn_layer_N, aggr=aggr,
                              relu=int(cfg.gnn_use_ReLU), layer_norm=int(cfg.use_feature_normalization),
-                             max_edge_dist=float(cfg.max_edge_dist))
+                             mapping=int(mapping), max_edge_dist=float(cfg.max_edge_dist))
         w = self._packed()
         aid = None
         if aggr == 0:

@@ -346,6 +346,9 @@ int fm_formation_stats_read(FmFormation* h, double* out_dev, int32_t clear, void
  *   adj       device [num_graphs / graphs_per_adj, E, E]: graph m reads matrix m / graphs_per_adj
  *   agent_id  device int32 [num_graphs] node gathered when aggr == 0 (NULL: m % graphs_per_adj)
  *   out       device [num_graphs, 16]
+ * Two kernel mappings compute it (fm_policy.cu): one WARP per graph (gnn_kernel<E, RELU>, compiled for the E values of
+ * FM_GNN_CASES), and one CTA per graph (gnn_wide_kernel<EMAX, RELU>, EMAX 32 or 64) for any 2 <= E <= 64 known at run
+ * time.  Both are fp32, deterministic and batch-invariant; they may differ from each other in the last bits.
  */
 typedef struct FmGnnConfig {
   int32_t num_graphs, graphs_per_adj, num_entities, node_feat_dim;
@@ -354,11 +357,16 @@ typedef struct FmGnnConfig {
   int32_t aggr;             /* 0 node gather, 1 global mean, 2 global max, 3 global add */
   int32_t relu;             /* 1 ReLU, 0 Tanh (embed_use_ReLU == gnn_use_ReLU) */
   int32_t layer_norm;       /* use_feature_normalization */
-  int32_t reserved_;
+  int32_t mapping;          /* 0 auto (= fm_gnn_mapping), 1 warp per graph (FM_ERR_UNSUPPORTED where E is not compiled),
+                               2 CTA per graph (any 2 <= E <= 64); anything else FM_ERR_INVALID_ARG */
   double max_edge_dist;
 } FmGnnConfig;
 int64_t fm_gnn_weight_floats(const FmGnnConfig* cfg);
-int fm_gnn_supported(int32_t num_entities, int32_t node_feat_dim);   /* 1 if the kernel is compiled for this graph size */
+/* 1 if the warp-per-graph kernel (mapping 1) is compiled for this graph size */
+int fm_gnn_supported(int32_t num_entities, int32_t node_feat_dim);
+/* the mapping that auto (0) selects for this graph size: 1 where the warp-per-graph kernel is compiled, else 2 for
+ * 2 <= E <= 64; 0 when no fused kernel covers it (E < 2, E > 64, or node_feat_dim outside 2..17) */
+int fm_gnn_mapping(int32_t num_entities, int32_t node_feat_dim);
 int fm_gnn_forward(int device, const FmGnnConfig* cfg, const float* weights, const float* node_obs, const float* adj,
                    const int32_t* agent_id, float* out, void* stream);
 
