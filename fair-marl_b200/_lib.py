@@ -87,6 +87,11 @@ class FmHeadConfig(C.Structure):
                 ("feature_norm", C.c_int32), ("relu", C.c_int32), ("num_outputs", C.c_int32), ("reserved_", C.c_int32)]
 
 
+class FmCriticHeadConfig(C.Structure):
+    _fields_ = [("num_rows", C.c_int32), ("cent_dim", C.c_int32), ("rows_per_env", C.c_int32), ("nbd_dim", C.c_int32),
+                ("layers", C.c_int32), ("recurrent", C.c_int32), ("feature_norm", C.c_int32), ("relu", C.c_int32)]
+
+
 class FairMarlError(RuntimeError):
     pass
 
@@ -153,6 +158,9 @@ def load():
         "fm_gnn_forward": ([C.c_int, C.POINTER(FmGnnConfig), vp, vp, vp, vp, vp, vp], C.c_int),
         "fm_head_weight_floats": ([C.POINTER(FmHeadConfig)], i64),
         "fm_policy_head": ([C.c_int, C.POINTER(FmHeadConfig), vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp], C.c_int),
+        "fm_gnn_gather": ([C.c_int, C.POINTER(FmGnnConfig), i32, vp, vp, vp, vp, vp, vp], C.c_int),
+        "fm_critic_head_weight_floats": ([C.POINTER(FmCriticHeadConfig)], i64),
+        "fm_critic_head": ([C.c_int, C.POINTER(FmCriticHeadConfig), vp, vp, vp, vp, vp, vp, vp, vp], C.c_int),
     }
     for name, (argtypes, restype) in sig.items():
         fn = getattr(lib, name)          # AttributeError if the .so does not export the ABI
@@ -170,7 +178,7 @@ EXPORTED_SYMBOLS = (
     "fm_formation_set_state",
     "fm_formation_get_state", "fm_formation_stats_enable", "fm_formation_stats_read", "fm_gnn_weight_floats", "fm_gnn_supported", "fm_gnn_mapping",
     "fm_gnn_forward",
-    "fm_head_weight_floats", "fm_policy_head",
+    "fm_head_weight_floats", "fm_policy_head", "fm_gnn_gather", "fm_critic_head_weight_floats", "fm_critic_head",
 )
 
 

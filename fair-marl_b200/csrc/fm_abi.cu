@@ -1201,7 +1201,30 @@ int fm_gnn_forward(int device, const FmGnnConfig* cfg, const float* weights, con
     return fail(FM_ERR_UNSUPPORTED, "fm_gnn_forward: embed_layers %d / conv_layers %d / aggr %d", cfg->embed_layers, cfg->conv_layers, cfg->aggr);
   int rc = use_device(device);
   if (rc) return rc;
-  FM_CUDA(fm::launch_gnn(*cfg, weights, node_obs, adj, agent_id, out, (cudaStream_t)stream));
+  FM_CUDA(fm::launch_gnn(*cfg, weights, node_obs, adj, agent_id, out, 0, (cudaStream_t)stream));
+  return FM_OK;
+}
+
+int fm_gnn_gather(int device, const FmGnnConfig* cfg, int32_t k, const float* weights, const float* node_obs,
+                  const float* adj, const int32_t* agent_id, float* out, void* stream) {
+  if (!cfg || !weights || !node_obs || !adj || !agent_id || !out) return fail(FM_ERR_INVALID_ARG, "fm_gnn_gather: null argument");
+  if (cfg->aggr != 0) return fail(FM_ERR_INVALID_ARG, "fm_gnn_gather: aggr %d (the gather is a node aggregation: 0)", cfg->aggr);
+  if (k < 1 || k > cfg->num_entities)
+    return fail(FM_ERR_INVALID_ARG, "fm_gnn_gather: k %d nodes per graph (1..%d)", k, cfg->num_entities);
+  if (cfg->num_graphs < 0 || cfg->graphs_per_adj < 1) return fail(FM_ERR_INVALID_ARG, "fm_gnn_gather: bad graph counts");
+  if (cfg->mapping < 0 || cfg->mapping > 2)
+    return fail(FM_ERR_INVALID_ARG, "fm_gnn_gather: mapping %d (0 auto, 1 warp per graph, 2 CTA per graph)", cfg->mapping);
+  const int E = cfg->num_entities, NF = cfg->node_feat_dim;
+  const bool ok = cfg->mapping == 0 ? fm_gnn_mapping(E, NF) != 0
+                : cfg->mapping == 1 ? fm_gnn_supported(E, NF) != 0
+                                    : fm::gnn_wide_supported_entities(E) && NF >= 2 && NF <= 17;
+  if (!ok)
+    return fail(FM_ERR_UNSUPPORTED, "fm_gnn_gather: mapping %d is not available for %d entities x %d features", cfg->mapping, E, NF);
+  if (cfg->embed_layers < 0 || cfg->embed_layers > 2 || cfg->conv_layers < 1 || cfg->conv_layers > 8)
+    return fail(FM_ERR_UNSUPPORTED, "fm_gnn_gather: embed_layers %d / conv_layers %d", cfg->embed_layers, cfg->conv_layers);
+  int rc = use_device(device);
+  if (rc) return rc;
+  FM_CUDA(fm::launch_gnn(*cfg, weights, node_obs, adj, agent_id, out, k, (cudaStream_t)stream));
   return FM_OK;
 }
 
@@ -1221,6 +1244,30 @@ int fm_policy_head(int device, const FmHeadConfig* cfg, const float* weights, co
   int rc = use_device(device);
   if (rc) return rc;
   FM_CUDA(fm::launch_head(*cfg, weights, obs, nbd, rnn_in, mask, u, rnn_out, logp, (long long*)action, value, (cudaStream_t)stream));
+  return FM_OK;
+}
+
+int64_t fm_critic_head_weight_floats(const FmCriticHeadConfig* cfg) {
+  if (!cfg) return 0;
+  return fm::critic_head_weight_count(cfg->cent_dim + cfg->nbd_dim, cfg->layers, cfg->recurrent);
+}
+
+int fm_critic_head(int device, const FmCriticHeadConfig* cfg, const float* weights, const float* cent_obs, const float* nbd,
+                   const float* rnn_in, const float* mask, float* rnn_out, float* value, void* stream) {
+  if (!cfg || !weights || !nbd || !value) return fail(FM_ERR_INVALID_ARG, "fm_critic_head: null argument");
+  if (cfg->num_rows < 0 || cfg->cent_dim < 0 || cfg->nbd_dim < 1 || (cfg->cent_dim > 0 && !cent_obs))
+    return fail(FM_ERR_INVALID_ARG, "fm_critic_head: num_rows %d / cent_dim %d (with cent_obs) / nbd_dim %d", cfg->num_rows,
+                cfg->cent_dim, cfg->nbd_dim);
+  if (cfg->cent_dim > 0 && (cfg->rows_per_env < 1 || cfg->num_rows % cfg->rows_per_env != 0))
+    return fail(FM_ERR_INVALID_ARG, "fm_critic_head: %d rows are not a whole number of envs of %d rows", cfg->num_rows, cfg->rows_per_env);
+  if ((int64_t)cfg->cent_dim + cfg->nbd_dim > fm::CRITIC_HEAD_MAX_IN)
+    return fail(FM_ERR_UNSUPPORTED, "fm_critic_head: %lld input features (at most %d)", (long long)cfg->cent_dim + cfg->nbd_dim,
+                fm::CRITIC_HEAD_MAX_IN);
+  if (cfg->layers < 0 || cfg->layers > 2) return fail(FM_ERR_UNSUPPORTED, "fm_critic_head: layers %d (0..2)", cfg->layers);
+  if (cfg->recurrent && (!rnn_in || !mask || !rnn_out)) return fail(FM_ERR_INVALID_ARG, "fm_critic_head: recurrent head needs rnn_in, mask, rnn_out");
+  int rc = use_device(device);
+  if (rc) return rc;
+  FM_CUDA(fm::launch_critic_head(*cfg, weights, cent_obs, nbd, rnn_in, mask, rnn_out, value, (cudaStream_t)stream));
   return FM_OK;
 }
 

@@ -95,12 +95,18 @@ bool gnn_supported_entities(int E);        // warp per graph (gnn_kernel<E, RELU
 constexpr int GNN_WIDE_MAX_ENTITIES = 2 * FM_MAX_AGENTS;
 bool gnn_wide_supported_entities(int E);   // CTA per graph (gnn_wide_kernel<EMAX, RELU>): 2 <= E <= 64
 int gnn_weight_count(int embed_layers, int conv_layers);
+// gather_k 0: aggr as in FmGnnConfig (gnn_kernel / gnn_wide_kernel); gather_k >= 1: the final states of gather_k nodes per
+// graph side by side (the GATHER instantiations, agent_id [M, gather_k])
 cudaError_t launch_gnn(const FmGnnConfig& c, const float* weights, const float* node, const float* adj, const int* agent_id,
-                       float* out, cudaStream_t st);
+                       float* out, int gather_k, cudaStream_t st);
 int head_weight_count(int layers, int recurrent);
 cudaError_t launch_head(const FmHeadConfig& c, const float* weights, const float* obs, const float* nbd, const float* rnn_in,
                         const float* mask, const float* u, float* rnn_out, float* logp, long long* action, float* value,
                         cudaStream_t st);
+constexpr int CRITIC_HEAD_MAX_IN = 768;    // critic_head_kernel: input width cap
+int critic_head_weight_count(int in_dim, int layers, int recurrent);
+cudaError_t launch_critic_head(const FmCriticHeadConfig& c, const float* weights, const float* cent_obs, const float* nbd,
+                               const float* rnn_in, const float* mask, float* rnn_out, float* value, cudaStream_t st);
 int formation_max_agents();
 int set_error(int code, const char* fmt, ...);   // fm_last_error text (fm_abi.cu)
 }  // namespace fm

@@ -91,7 +91,10 @@ struct GnnLayout {
   static constexpr int WORDS = (END + 3) & ~3;                // floats per warp
 };
 
-template <int E, bool RELU>
+// GATHER (a template parameter on the epilogue only, so that the instantiations without it keep their code): the final
+// states of k = a.aggr nodes per graph side by side (agent_id [M, k] -> out [M, k * 16]).  Otherwise aggr selects one node
+// (agent_id [M]) or a global pool.
+template <int E, bool RELU, bool GATHER = false>
 __global__ void __launch_bounds__(G_WARPS * 32, 2) gnn_kernel(const __grid_constant__ GnnArgs a) {
   using L = GnnLayout<E>;
   constexpr int LPT = L::LPT, SPL = L::SPL;
@@ -350,7 +353,13 @@ __global__ void __launch_bounds__(G_WARPS * 32, 2) gnn_kernel(const __grid_const
       __syncwarp();
     }
     // ---- aggregation ----------------------------------------------------------------------------------------
-    if (lane < GH) {
+    if constexpr (GATHER) {
+      const int k = a.aggr;
+      for (int o = lane; o < k * GH; o += 32) {
+        const int node = a.agent_id[(size_t)m * k + (o >> 4)];
+        a.out[(size_t)m * k * GH + o] = s_x[min(max(node, 0), E - 1) * GXS + (o & 15)];
+      }
+    } else if (lane < GH) {
       float v;
       if (a.aggr == 0) {
         const int node = a.agent_id ? a.agent_id[m] : (m % a.rep);
@@ -367,7 +376,7 @@ __global__ void __launch_bounds__(G_WARPS * 32, 2) gnn_kernel(const __grid_const
 }
 
 template <int E>
-static cudaError_t gnn_launch_e(const GnnArgs& a, cudaStream_t st) {
+static cudaError_t gnn_launch_e(const GnnArgs& a, int k, cudaStream_t st) {
   using L = GnnLayout<E>;
   const size_t smem = (size_t)(((a.wfloats + 3) & ~3) + G_WARPS * L::WORDS) * sizeof(float);
   int dev = 0, sms = 0;
@@ -376,7 +385,14 @@ static cudaError_t gnn_launch_e(const GnnArgs& a, cudaStream_t st) {
   if (e != cudaSuccess) return e;
   const int want = (a.M + G_WARPS - 1) / G_WARPS;
   const int grid = want < 2 * sms ? want : 2 * sms;
-  if (a.relu) {
+  if (k > 0) {                                                // multi-node gather: aggr carries k
+    GnnArgs g = a;
+    g.aggr = k;
+    const auto kern = a.relu ? gnn_kernel<E, true, true> : gnn_kernel<E, false, true>;
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<grid, G_WARPS * 32, smem, st>>>(g);
+  } else if (a.relu) {
     e = cudaFuncSetAttribute(gnn_kernel<E, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     gnn_kernel<E, true><<<grid, G_WARPS * 32, smem, st>>>(a);
@@ -405,7 +421,7 @@ __host__ __device__ inline int gnn_wide_scratch_floats(int E) {
   return ((E * E + 3) & ~3) + E * (GnnLayout<1>::NFP + GXS + GQS);
 }
 
-template <int EMAX, bool RELU>
+template <int EMAX, bool RELU, bool GATHER = false>        // GATHER: as in gnn_kernel
 __global__ void __launch_bounds__(GW_THREADS, 2) gnn_wide_kernel(const __grid_constant__ GnnArgs a, const int E) {
   constexpr int P = GW_THREADS / EMAX;                        // threads per target
   constexpr int SPL = EMAX / P;                               // sources per thread (at most)
@@ -664,7 +680,13 @@ __global__ void __launch_bounds__(GW_THREADS, 2) gnn_wide_kernel(const __grid_co
       __syncthreads();                                        // s_x complete; s_q free for the next layer
     }
     // ---- aggregation ----------------------------------------------------------------------------------------
-    if (tid < GH) {
+    if constexpr (GATHER) {
+      const int k = a.aggr;
+      for (int o = tid; o < k * GH; o += GW_THREADS) {
+        const int node = a.agent_id[(size_t)m * k + (o >> 4)];
+        a.out[(size_t)m * k * GH + o] = s_x[min(max(node, 0), E - 1) * GXS + (o & 15)];
+      }
+    } else if (tid < GH) {
       float v;
       if (a.aggr == 0) {
         const int node = a.agent_id ? a.agent_id[m] : (m % a.rep);
@@ -681,25 +703,32 @@ __global__ void __launch_bounds__(GW_THREADS, 2) gnn_wide_kernel(const __grid_co
 }
 
 template <int EMAX, bool RELU>
-static cudaError_t gnn_wide_launch_k(const GnnArgs& a, int E, size_t smem, int sms, cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute(gnn_wide_kernel<EMAX, RELU>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+static cudaError_t gnn_wide_launch_k(const GnnArgs& a, int E, int k, size_t smem, int sms, cudaStream_t st) {
+  const void* kern = k > 0 ? (const void*)gnn_wide_kernel<EMAX, RELU, true> : (const void*)gnn_wide_kernel<EMAX, RELU>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   int per_sm = 0;
-  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, gnn_wide_kernel<EMAX, RELU>, GW_THREADS, smem);
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, GW_THREADS, smem);
   if (e != cudaSuccess) return e;
   if (per_sm < 1) return cudaErrorInvalidConfiguration;
   const int grid = a.M < per_sm * sms ? a.M : per_sm * sms;
-  gnn_wide_kernel<EMAX, RELU><<<grid, GW_THREADS, smem, st>>>(a, E);
+  if (k > 0) {                                                // multi-node gather: aggr carries k
+    GnnArgs g = a;
+    g.aggr = k;
+    gnn_wide_kernel<EMAX, RELU, true><<<grid, GW_THREADS, smem, st>>>(g, E);
+  } else {
+    gnn_wide_kernel<EMAX, RELU><<<grid, GW_THREADS, smem, st>>>(a, E);
+  }
   return cudaGetLastError();
 }
 
-static cudaError_t gnn_wide_launch(const GnnArgs& a, int E, cudaStream_t st) {
+static cudaError_t gnn_wide_launch(const GnnArgs& a, int E, int k, cudaStream_t st) {
   const size_t smem = (size_t)(((a.wfloats + 3) & ~3) + gnn_wide_scratch_floats(E)) * sizeof(float);
   int dev = 0, sms = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   if (e != cudaSuccess) return e;
-  if (E <= 32) return a.relu ? gnn_wide_launch_k<32, true>(a, E, smem, sms, st) : gnn_wide_launch_k<32, false>(a, E, smem, sms, st);
-  return a.relu ? gnn_wide_launch_k<64, true>(a, E, smem, sms, st) : gnn_wide_launch_k<64, false>(a, E, smem, sms, st);
+  if (E <= 32) return a.relu ? gnn_wide_launch_k<32, true>(a, E, k, smem, sms, st) : gnn_wide_launch_k<32, false>(a, E, k, smem, sms, st);
+  return a.relu ? gnn_wide_launch_k<64, true>(a, E, k, smem, sms, st) : gnn_wide_launch_k<64, false>(a, E, k, smem, sms, st);
 }
 
 // E values compiled: the navigation / formation shapes at N = 2..7 with O <= 3 and up to 2 walls
@@ -715,7 +744,7 @@ bool gnn_supported_entities(int E) {
 bool gnn_wide_supported_entities(int E) { return E >= 2 && E <= GNN_WIDE_MAX_ENTITIES; }
 
 cudaError_t launch_gnn(const FmGnnConfig& c, const float* weights, const float* node, const float* adj, const int* agent_id,
-                       float* out, cudaStream_t st) {
+                       float* out, int gather_k, cudaStream_t st) {
   GnnArgs a;
   a.w = weights; a.node = node; a.adj = adj; a.agent_id = agent_id; a.out = out;
   a.M = c.num_graphs; a.rep = c.graphs_per_adj; a.NF = c.node_feat_dim; a.embed_layers = c.embed_layers;
@@ -724,9 +753,9 @@ cudaError_t launch_gnn(const FmGnnConfig& c, const float* weights, const float* 
   a.wfloats = gnn_weight_floats(c.embed_layers, c.conv_layers);
   if (a.M <= 0) return cudaSuccess;
   const int mapping = c.mapping != 0 ? c.mapping : (gnn_supported_entities(c.num_entities) ? 1 : 2);
-  if (mapping == 2) return gnn_wide_supported_entities(c.num_entities) ? gnn_wide_launch(a, c.num_entities, st) : cudaErrorInvalidValue;
+  if (mapping == 2) return gnn_wide_supported_entities(c.num_entities) ? gnn_wide_launch(a, c.num_entities, gather_k, st) : cudaErrorInvalidValue;
   if (mapping != 1) return cudaErrorInvalidValue;
-#define X(e) if (c.num_entities == e) return gnn_launch_e<e>(a, st);
+#define X(e) if (c.num_entities == e) return gnn_launch_e<e>(a, gather_k, st);
   FM_GNN_CASES(X)
 #undef X
   return cudaErrorInvalidValue;
@@ -952,6 +981,193 @@ cudaError_t launch_head(const FmHeadConfig& c, const float* weights, const float
     if (e != cudaSuccess) return e;
     head_kernel<false><<<grid, HEAD_WARPS * 32, smem, st>>>(a);
   }
+  return cudaGetLastError();
+}
+
+// =====================================================================================================================
+// Fused CRITIC head for wide inputs: GR_Critic.forward after gnn_base (graph_actor_critic.py:323-397) on
+// x = [cent_obs | nbd] of D = cent_dim + nbd_dim <= CRITIC_HEAD_MAX_IN features, where head_kernel (D <= 32) cannot serve:
+// use_cent_obs (cent_obs = share_obs, the N agents' observations side by side) and critic_graph_aggr = 'node' (nbd = the
+// N agent nodes' features side by side, fm_gnn_gather).  Same function as head_kernel with the value layer: feature
+// LayerNorm over all D inputs -> MLPBase -> one GRU step -> v_out.
+// fc1 at D = 736 is 184 KB of weights and the GRU 97.5 KB: together they do not fit a block's shared memory, so fc1 stays
+// in global memory (L2) and is amortised over a tile of rows instead:
+//   one WARP per tile of CH_ROWS consecutive rows (persistent); lane l owns hidden units l and l + 32, as in head_kernel;
+//   the feature-LayerNorm statistics of each row over all D inputs (two passes: mean, then the centred variance);
+//   fc1 over K-chunks of 32 inputs: the chunk of the tile's rows is normalised into a warp-private scratch, and each k-quad
+//   of the lane's two weight columns is read once (two LDG.128) for all CH_ROWS rows;
+//   everything after fc1 one row at a time, with the weights in shared memory, as head_kernel.
+// The cent_obs part of a row is read from the env-level slab [M / rows_per_env, cent_dim] (row m: env m / rows_per_env).
+// Every row is computed by one warp in a fixed order that does not depend on the tile it falls in: deterministic and
+// batch-invariant, no atomics.
+constexpr int CH_WARPS = 16;
+constexpr int CH_ROWS = 8;                               // rows per warp tile
+constexpr int CH_SCRATCH = CH_ROWS * HH + 2 * HH;        // per warp: fc1 chunk / fc1 outputs [CH_ROWS][64] | xs[64] | hs[64]
+
+__host__ __device__ inline int critic_head_pad(int in_dim) { return (in_dim + 31) & ~31; }
+
+__host__ __device__ inline int critic_head_tail_floats(int layers, int recurrent) {
+  return 3 * HH + layers * HW_FC_SZ + (recurrent ? HW_GRU_SZ : 0) + HW_OUT_SZ;
+}
+
+__host__ __device__ inline int critic_head_weight_floats(int in_dim, int layers, int recurrent) {
+  const int Dp = critic_head_pad(in_dim);
+  return 2 * Dp + Dp * HH + critic_head_tail_floats(layers, recurrent);
+}
+
+struct CriticHeadArgs {
+  const float* w;
+  const float* cent;       // [M / rows_per_env, cent_dim] or null (cent_dim 0)
+  const float* nbd;        // [M, nbd_dim]
+  const float* rnn_in;     // [M, 64]   (recurrent)
+  const float* mask;       // [M]       (recurrent)
+  float* rnn_out;          // [M, 64]   (recurrent)
+  float* value;            // [M]
+  int M, cent_dim, rows_per_env, nbd_dim, layers, recurrent, feat_norm;
+};
+
+template <bool RELU>
+__global__ void __launch_bounds__(CH_WARPS * 32, 1) critic_head_kernel(const __grid_constant__ CriticHeadArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  const int D = a.cent_dim + a.nbd_dim, Dp = critic_head_pad(D);
+  const int tail = critic_head_tail_floats(a.layers, a.recurrent);
+  float* Wfn = smem;                                         // feature_norm gamma[Dp] | beta[Dp]
+  float* Wt = smem + 2 * Dp;                                 // fc1 b | ln gamma | ln beta, hidden layers, GRU, output
+  const float* fc1 = a.w + 2 * Dp;                           // [Dp / 4][64][4] in global memory
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  float* xr = smem + ((2 * Dp + tail + 3) & ~3) + wib * CH_SCRATCH;
+  float* xs = xr + CH_ROWS * HH;
+  float* hs = xs + HH;
+  for (int k = threadIdx.x; k < 2 * Dp; k += blockDim.x) Wfn[k] = __ldg(a.w + k);
+  for (int k = threadIdx.x; k < tail; k += blockDim.x) Wt[k] = __ldg(fc1 + (size_t)Dp * HH + k);
+  __syncthreads();
+  const float* w_gru = Wt + 3 * HH + a.layers * HW_FC_SZ;
+  const float* w_out = w_gru + (a.recurrent ? HW_GRU_SZ : 0);
+  const int c2[2] = {lane, lane + 32};
+  const int cd = a.cent_dim;
+  auto in = [&](int m, int k) -> float {                    // x[m][k], k < D
+    return k < cd ? __ldg(a.cent + (size_t)(m / a.rows_per_env) * cd + k) : __ldg(a.nbd + (size_t)m * a.nbd_dim + (k - cd));
+  };
+  const int tiles = (a.M + CH_ROWS - 1) / CH_ROWS;
+  for (int tile = blockIdx.x * CH_WARPS + wib; tile < tiles; tile += gridDim.x * CH_WARPS) {
+    const int m0 = tile * CH_ROWS;
+    const int nr = min(CH_ROWS, a.M - m0);
+    // ---- feature LayerNorm statistics over all D inputs of each row ----------------------------------------------------
+    float mean[CH_ROWS], inv[CH_ROWS];
+#pragma unroll
+    for (int r = 0; r < CH_ROWS; ++r) {
+      mean[r] = 0.f; inv[r] = 1.f;
+      if (a.feat_norm && r < nr) {
+        float sum = 0.f;
+        for (int k = lane; k < D; k += 32) sum += in(m0 + r, k);
+        const float mu = warp_sum(sum) / (float)D;
+        float q = 0.f;
+        for (int k = lane; k < D; k += 32) { const float d = in(m0 + r, k) - mu; q = fmaf(d, d, q); }
+        mean[r] = mu;
+        inv[r] = rsqrtf(warp_sum(q) / (float)D + 1e-5f);
+      }
+    }
+    // ---- fc1 over K-chunks of 32 inputs, the weights of a chunk read once for the tile ----------------------------------
+    float acc[CH_ROWS][2];
+#pragma unroll
+    for (int r = 0; r < CH_ROWS; ++r) { acc[r][0] = Wt[lane]; acc[r][1] = Wt[lane + 32]; }
+    for (int k0 = 0; k0 < Dp; k0 += 32) {
+      const int k = k0 + lane;
+#pragma unroll
+      for (int r = 0; r < CH_ROWS; ++r) {
+        float x = 0.f;
+        if (r < nr && k < D) {
+          x = in(m0 + r, k);
+          if (a.feat_norm) x = fmaf((x - mean[r]) * inv[r], Wfn[k], Wfn[Dp + k]);
+        }
+        xr[r * 32 + lane] = x;
+      }
+      __syncwarp();
+      const float4* wq = reinterpret_cast<const float4*>(fc1 + (size_t)k0 * HH);
+#pragma unroll 2
+      for (int q = 0; q < 8; ++q) {
+        const float4 w0 = __ldg(wq + q * HH + lane), w1 = __ldg(wq + q * HH + lane + 32);
+#pragma unroll
+        for (int r = 0; r < CH_ROWS; ++r) {
+          const float4 x4 = *reinterpret_cast<const float4*>(xr + r * 32 + 4 * q);
+          acc[r][0] = fmaf(w0.x, x4.x, acc[r][0]); acc[r][0] = fmaf(w0.y, x4.y, acc[r][0]);
+          acc[r][0] = fmaf(w0.z, x4.z, acc[r][0]); acc[r][0] = fmaf(w0.w, x4.w, acc[r][0]);
+          acc[r][1] = fmaf(w1.x, x4.x, acc[r][1]); acc[r][1] = fmaf(w1.y, x4.y, acc[r][1]);
+          acc[r][1] = fmaf(w1.z, x4.z, acc[r][1]); acc[r][1] = fmaf(w1.w, x4.w, acc[r][1]);
+        }
+      }
+      __syncwarp();
+    }
+#pragma unroll
+    for (int r = 0; r < CH_ROWS; ++r) { xr[r * HH + lane] = acc[r][0]; xr[r * HH + lane + 32] = acc[r][1]; }
+    __syncwarp();
+    // ---- the rest of the head, one row at a time (head_kernel's arithmetic) -------------------------------------------
+#pragma unroll 1
+    for (int r = 0; r < nr; ++r) {
+      const int m = m0 + r;
+      float h0 = g_act<RELU>(xr[r * HH + lane]), h1 = g_act<RELU>(xr[r * HH + lane + 32]);
+      head_ln(h0, h1, Wt + HH, lane);
+      xs[lane] = h0; xs[lane + 32] = h1;
+      __syncwarp();
+      for (int l = 0; l < a.layers; ++l) {
+        const float* wl = Wt + 3 * HH + l * HW_FC_SZ;
+        float hacc[2] = {wl[HH * HH + lane], wl[HH * HH + lane + 32]};
+        head_matvec<2>(wl, HH, HH / 4, xs, c2, hacc);
+        h0 = g_act<RELU>(hacc[0]); h1 = g_act<RELU>(hacc[1]);
+        head_ln(h0, h1, wl + HH * HH + HH, lane);
+        __syncwarp();
+        xs[lane] = h0; xs[lane + 32] = h1;
+        __syncwarp();
+      }
+      if (a.recurrent) {
+        const float mk = a.mask[m];
+        const float p0 = __ldcs(a.rnn_in + (size_t)m * HH + lane) * mk, p1 = __ldcs(a.rnn_in + (size_t)m * HH + lane + 32) * mk;
+        hs[lane] = p0; hs[lane + 32] = p1;
+        __syncwarp();
+        const int c6[6] = {lane, lane + 32, HH + lane, HH + lane + 32, 2 * HH + lane, 2 * HH + lane + 32};
+        const float* bih = w_gru + 2 * HH * 3 * HH;
+        const float* bhh = bih + 3 * HH;
+        float gi[6], gh[6];
+#pragma unroll
+        for (int c = 0; c < 6; ++c) { gi[c] = bih[c6[c]]; gh[c] = bhh[c6[c]]; }
+        head_matvec<6>(w_gru, 3 * HH, HH / 4, xs, c6, gi);
+        head_matvec<6>(w_gru + HH * 3 * HH, 3 * HH, HH / 4, hs, c6, gh);
+        const float r0 = 1.0f / (1.0f + expf(-(gi[0] + gh[0]))), r1 = 1.0f / (1.0f + expf(-(gi[1] + gh[1])));
+        const float z0 = 1.0f / (1.0f + expf(-(gi[2] + gh[2]))), z1 = 1.0f / (1.0f + expf(-(gi[3] + gh[3])));
+        const float n0 = tanhf(gi[4] + r0 * gh[4]), n1 = tanhf(gi[5] + r1 * gh[5]);
+        h0 = (1.0f - z0) * n0 + z0 * p0; h1 = (1.0f - z1) * n1 + z1 * p1;
+        a.rnn_out[(size_t)m * HH + lane] = h0; a.rnn_out[(size_t)m * HH + lane + 32] = h1;
+        head_ln(h0, h1, bhh + 3 * HH, lane);
+      }
+      const float v = warp_sum(fmaf(w_out[lane], h0, w_out[lane + 32] * h1)) + w_out[8 * HH];
+      if (lane == 0) a.value[m] = v;
+      __syncwarp();
+    }
+  }
+}
+
+int critic_head_weight_count(int in_dim, int layers, int recurrent) { return critic_head_weight_floats(in_dim, layers, recurrent); }
+
+cudaError_t launch_critic_head(const FmCriticHeadConfig& c, const float* weights, const float* cent_obs, const float* nbd,
+                               const float* rnn_in, const float* mask, float* rnn_out, float* value, cudaStream_t st) {
+  CriticHeadArgs a;
+  a.w = weights; a.cent = cent_obs; a.nbd = nbd; a.rnn_in = rnn_in; a.mask = mask; a.rnn_out = rnn_out; a.value = value;
+  a.M = c.num_rows; a.cent_dim = c.cent_dim; a.rows_per_env = c.rows_per_env; a.nbd_dim = c.nbd_dim; a.layers = c.layers;
+  a.recurrent = c.recurrent; a.feat_norm = c.feature_norm;
+  if (a.M <= 0) return cudaSuccess;
+  const int Dp = critic_head_pad(a.cent_dim + a.nbd_dim);
+  const size_t smem = (size_t)(((2 * Dp + critic_head_tail_floats(a.layers, a.recurrent) + 3) & ~3) + CH_WARPS * CH_SCRATCH) * sizeof(float);
+  int dev = 0, sms = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (e != cudaSuccess) return e;
+  const int tiles = (a.M + CH_ROWS - 1) / CH_ROWS;
+  const int want = (tiles + CH_WARPS - 1) / CH_WARPS;
+  const int grid = want < sms ? want : sms;
+  const auto kern = c.relu ? critic_head_kernel<true> : critic_head_kernel<false>;
+  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  kern<<<grid, CH_WARPS * 32, smem, st>>>(a);
   return cudaGetLastError();
 }
 

@@ -245,8 +245,9 @@ class DenseGNNBase(nn.Module):
     def forward_fused(self, node_obs: Tensor, adj_env: Tensor, graphs_per_adj: int, agent_id: Optional[Tensor],
                       mapping: int = 0) -> Tensor:
         """One launch of ``fm_gnn_forward``.  node_obs [M, E, F] contiguous fp32; adj_env [M / graphs_per_adj, E, E];
-        agent_id [M] or [M, 1] node indices (aggr 'node').  ``mapping``: 0 auto, 1 the warp-per-graph kernel, 2 the
-        CTA-per-graph kernel (``FmGnnConfig.mapping``)."""
+        agent_id [M] or [M, 1] node indices (aggr 'node'), or [M, k] with k > 1: the k nodes' features side by side
+        ([M, k * 16], ``fm_gnn_gather``).  ``mapping``: 0 auto, 1 the warp-per-graph kernel, 2 the CTA-per-graph kernel
+        (``FmGnnConfig.mapping``)."""
         import ctypes as C
         from fair_marl_b200 import _lib
         cfg = self.cfg
@@ -260,12 +261,19 @@ class DenseGNNBase(nn.Module):
                              mapping=int(mapping), max_edge_dist=float(cfg.max_edge_dist))
         w = self._packed()
         aid = None
+        stream = torch.cuda.current_stream(node_obs.device).cuda_stream
         if aggr == 0:
-            if agent_id is None or agent_id.numel() != M:
-                raise ValueError("forward_fused: aggr 'node' gathers ONE node per graph (agent_id [M])")
+            if agent_id is None or agent_id.numel() == 0 or agent_id.numel() % max(M, 1) != 0:
+                raise ValueError("forward_fused: aggr 'node' gathers k nodes per graph (agent_id [M] or [M, k])")
+            k = agent_id.numel() // max(M, 1)
+            if k > 1:
+                aid = agent_id.reshape(M, k).to(torch.int32).contiguous()
+                out = torch.empty((M, k * cfg.gnn_hidden_size), dtype=torch.float32, device=node_obs.device)
+                _lib.check(_lib.load().fm_gnn_gather(node_obs.device.index, C.byref(c), k, w.data_ptr(), node_obs.data_ptr(),
+                                                     adj_env.data_ptr(), aid.data_ptr(), out.data_ptr(), stream), "fm_gnn_gather")
+                return out
             aid = agent_id.reshape(M).to(torch.int32).contiguous()
         out = torch.empty((M, cfg.gnn_hidden_size), dtype=torch.float32, device=node_obs.device)
-        stream = torch.cuda.current_stream(node_obs.device).cuda_stream
         _lib.check(_lib.load().fm_gnn_forward(node_obs.device.index, C.byref(c), w.data_ptr(), node_obs.data_ptr(),
                                               adj_env.data_ptr(), aid.data_ptr() if aid is not None else None,
                                               out.data_ptr(), stream), "fm_gnn_forward")
@@ -274,8 +282,7 @@ class DenseGNNBase(nn.Module):
     def forward(self, node_obs: Tensor, adj: Tensor, agent_id: Tensor, adj_env: Optional[Tuple[Tensor, int]] = None) -> Tensor:
         """node_obs [M, E, F]; adj [M, E, E] (any stride, e.g. the env's matrix expanded over its agents);
         agent_id [M, k] integer node indices.  ``adj_env``: see the class docstring."""
-        if adj_env is not None and (self.graph_aggr != "node" or agent_id.numel() == node_obs.shape[0]) \
-                and self.fused_available(node_obs):
+        if adj_env is not None and self.fused_available(node_obs):
             return self.forward_fused(node_obs.contiguous(), adj_env[0], adj_env[1], agent_id)
         mask = edge_mask(adj, self.cfg.max_edge_dist)
         x = self.embed_layer(node_obs, adj, mask)
@@ -372,17 +379,19 @@ class _Trunk(nn.Module):
     def _out_linear(self) -> nn.Linear:
         raise NotImplementedError
 
-    def pack_head_weights(self) -> Tensor:
-        """The weight blob ``fm_policy_head`` reads (layout: include/fairmarl.h ``FmHeadConfig``)."""
+    def pack_head_weights(self, width: int = 32) -> Tensor:
+        """The weight blob ``fm_policy_head`` reads (layout: include/fairmarl.h ``FmHeadConfig``), or with ``width`` the
+        padded input width Dp of the blob ``fm_critic_head`` reads (``FmCriticHeadConfig``): the two differ only in the
+        width of the feature norm and of fc1."""
         base, dt = self.base, torch.float32
         dev = base.lins[0].weight.device
         D, H = self._head_in, 64
-        g, b = torch.ones(32, dtype=dt, device=dev), torch.zeros(32, dtype=dt, device=dev)
+        g, b = torch.ones(width, dtype=dt, device=dev), torch.zeros(width, dtype=dt, device=dev)
         if isinstance(base.feature_norm, nn.LayerNorm):
             g[:D], b[:D] = base.feature_norm.weight.detach().to(dt), base.feature_norm.bias.detach().to(dt)
         parts = [g, b]
         for k, (lin, norm) in enumerate(zip(base.lins, base.norms)):
-            parts += [_quad_interleave(lin.weight.detach().to(dt).t(), 32 if k == 0 else H), lin.bias.detach().to(dt),
+            parts += [_quad_interleave(lin.weight.detach().to(dt).t(), width if k == 0 else H), lin.bias.detach().to(dt),
                       norm.weight.detach().to(dt), norm.bias.detach().to(dt)]
         if self.recurrent:
             r = self.rnn.rnn
@@ -395,11 +404,11 @@ class _Trunk(nn.Module):
         parts += [wo.reshape(-1), bo]
         return torch.cat([x.reshape(-1) for x in parts]).contiguous()
 
-    def _packed_head(self) -> Tensor:
+    def _packed_head(self, width: int = 32) -> Tensor:
         ps = [p for n, p in self.named_parameters() if not n.startswith("gnn_base.")]
-        key = tuple((p.data_ptr(), p._version) for p in ps)
+        key = (width,) + tuple((p.data_ptr(), p._version) for p in ps)
         if getattr(self, "_head_key", None) != key:
-            self._head_key, self._head_pack = key, self.pack_head_weights()
+            self._head_key, self._head_pack = key, self.pack_head_weights(width)
         return self._head_pack
 
     def _run_head(self, obs: Optional[Tensor], nbd: Tensor, rnn_states: Tensor, masks: Tensor, u: Optional[Tensor], critic: bool):
@@ -485,13 +494,65 @@ class DenseGraphCritic(_Trunk):
     def _out_linear(self) -> nn.Linear:
         return self.v_out
 
+    # fm_critic_head's input width cap (csrc/fm_launch.h CRITIC_HEAD_MAX_IN)
+    CRITIC_HEAD_MAX_IN = 768
+
+    def critic_head_supported(self) -> bool:
+        """The fused heads cover this critic: ``fm_policy_head`` for inputs of at most 32 features, ``fm_critic_head``
+        above that, up to CRITIC_HEAD_MAX_IN."""
+        cfg = self.cfg
+        return (cfg.hidden_size == 64 and cfg.layer_N <= 2 and self.gnn_base.out_dim == 16 and self._head_in <= self.CRITIC_HEAD_MAX_IN
+                and (not self.recurrent or cfg.recurrent_N == 1))
+
+    def _run_critic_head(self, cent: Optional[Tuple[Tensor, int]], nbd: Tensor, rnn_states: Tensor, masks: Tensor):
+        """One launch of ``fm_critic_head``: cent = (cent_obs [M / rows_per_env, cent_dim], rows_per_env) or None; nbd
+        [M, nbd_dim] -> (values [M, 1], rnn_states)."""
+        import ctypes as C
+        from fair_marl_b200 import _lib
+        cfg = self.cfg
+        M, dev = nbd.shape[0], nbd.device
+        cent_obs = cent[0].contiguous() if cent is not None else None
+        c = _lib.FmCriticHeadConfig(num_rows=M, cent_dim=0 if cent is None else cent_obs.shape[1],
+                                    rows_per_env=1 if cent is None else int(cent[1]), nbd_dim=nbd.shape[1], layers=cfg.layer_N,
+                                    recurrent=int(self.recurrent), feature_norm=int(cfg.use_feature_normalization),
+                                    relu=int(cfg.use_ReLU))
+        if cent is not None and cent_obs.shape[0] * c.rows_per_env != M:
+            raise ValueError("_run_critic_head: cent_obs must hold one row per rows_per_env rows")
+        w = self._packed_head((self._head_in + 31) // 32 * 32)
+        nbd = nbd.contiguous()
+        rnn_in = rnn_states.reshape(M, -1).contiguous() if self.recurrent else None
+        rnn_out = torch.empty((M, 1, 64), dtype=torch.float32, device=dev) if self.recurrent else rnn_states
+        mk = masks.reshape(M).to(torch.float32).contiguous() if self.recurrent else None
+        value = torch.empty((M, 1), dtype=torch.float32, device=dev)
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        _lib.check(_lib.load().fm_critic_head(dev.index, C.byref(c), w.data_ptr(), ptr(cent_obs), nbd.data_ptr(), ptr(rnn_in),
+                                              ptr(mk), ptr(rnn_out) if self.recurrent else None, value.data_ptr(),
+                                              torch.cuda.current_stream(dev).cuda_stream), "fm_critic_head")
+        return value, rnn_out
+
     def forward(self, cent_obs: Optional[Tensor], node_obs: Tensor, adj: Tensor, agent_id: Tensor, rnn_states: Tensor,
-                masks: Tensor, adj_env: Optional[Tuple[Tensor, int]] = None) -> Tuple[Tensor, Tensor]:
-        if (adj_env is not None and not self.cfg.use_cent_obs and self.cfg.critic_graph_aggr != "node" and self.head_supported()
-                and self.gnn_base.fused_available(node_obs)):
-            nbd = self.gnn_base.forward_fused(node_obs.contiguous(), adj_env[0], adj_env[1], None)
-            return self._run_head(None, nbd, rnn_states, masks, None, critic=True)
+                masks: Tensor, adj_env: Optional[Tuple[Tensor, int]] = None,
+                cent_env: Optional[Tuple[Tensor, int]] = None) -> Tuple[Tensor, Tensor]:
+        """cent_obs [M, N * obs_dim] (use_cent_obs; ``share_obs``) or, without a per-row copy, ``cent_env =
+        (obs [M / rows_per_env, N * obs_dim], rows_per_env)``: one row per env, read by its rows_per_env ego graphs, as
+        ``adj_env`` passes the adjacency.  agent_id [M, 1], or [M, N] (``share_agent_id``) for critic_graph_aggr='node'.
+        With ``adj_env`` and a covered configuration (``critic_head_supported``) this is two launches: the fused graph
+        network (a k-node gather for 'node') and the fused head, chosen by the input width D: ``fm_policy_head`` for
+        D <= 32, ``fm_critic_head`` above.  Otherwise the dense modules."""
+        cent = None
+        if self.cfg.use_cent_obs:
+            cent = cent_env if cent_env is not None else (cent_obs, 1)
+        if adj_env is not None and self.critic_head_supported() and self.gnn_base.fused_available(node_obs):
+            nbd = self.gnn_base.forward_fused(node_obs.contiguous(), adj_env[0], adj_env[1],
+                                              agent_id if self.cfg.critic_graph_aggr == "node" else None)
+            if self._head_in > 32:
+                return self._run_critic_head(cent, nbd, rnn_states, masks)
+            x = nbd if cent is None else torch.cat([cent[0].repeat_interleave(cent[1], dim=0), nbd], dim=1)
+            D = x.shape[1]
+            return self._run_head(x[:, :D - 16] if D > 16 else None, x[:, D - 16:].contiguous(), rnn_states, masks, None, critic=True)
         nbd = self.gnn_base(node_obs, adj, agent_id, adj_env=adj_env)
+        if cent is not None and cent_obs is None:
+            cent_obs = cent[0].repeat_interleave(cent[1], dim=0)
         x = torch.cat([cent_obs, nbd], dim=1) if self.cfg.use_cent_obs else nbd
         x = self.base(x)
         if self.recurrent:

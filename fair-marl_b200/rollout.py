@@ -152,12 +152,25 @@ class RolloutCollector:
         E = env.num_entities
         self.fused = bool(fused) if fused is not None else (
             env.device.type == "cuda" and fused_gnn_supported(actor.cfg, E, actor.gnn_base.graph_aggr)
-            and fused_gnn_supported(critic.cfg, E, critic.gnn_base.graph_aggr)
-            and not (critic.cfg.critic_graph_aggr == "node"))
-        if cfg.use_cent_obs or critic.cfg.critic_graph_aggr == "node":
-            # GR_Critic concatenates cent_obs / gathers the N agents' rows via share_agent_id (graph_actor_critic.py:323-397);
-            # this loop feeds neither (ADVICE r1): refuse instead of crashing inside the MLP
-            raise NotImplementedError("RolloutCollector: use_cent_obs / critic_graph_aggr='node' are not wired into the device loop")
+            and fused_gnn_supported(critic.cfg, E, critic.gnn_base.graph_aggr))
+
+    def _critic_inputs(self, t: int, lo: int, hi: int):
+        """What GMPERunner.collect feeds GR_Critic for rows lo:hi of slab t (graph_mpe_runner.py:396-436): share_obs
+        (use_cent_obs) and share_agent_id (critic_graph_aggr='node', else agent_id) -> (cent_obs, agent_id, cent_env).
+        The fused critic reads share_obs as the env-level slab (cent_env, no per-row copy); the dense one gets rows."""
+        b, ccfg = self.buffer, self.critic.cfg
+        N = b.num_agents
+        if ccfg.critic_graph_aggr == "node":
+            aid = b.share_agent_id[t][lo // N:hi // N].reshape(hi - lo, N)
+        else:
+            aid = b.agent_id[t][lo // N:hi // N].reshape(hi - lo, 1)
+        cent_obs = cent_env = None
+        if ccfg.use_cent_obs:
+            if self.fused:
+                cent_env = (b.obs[t][lo // N:hi // N].reshape(-1, N * b.obs.shape[-1]), N)
+            else:
+                cent_obs = b.share_obs[t][lo // N:hi // N].reshape(hi - lo, -1)
+        return cent_obs, aid, cent_env
 
     def warmup(self) -> None:
         """``GMPERunner.warmup`` (:178-203): reset the envs; the observation lands in slab 0."""
@@ -184,7 +197,8 @@ class RolloutCollector:
             adj_e = (b.adj_env[t][lo // N:hi // N], N) if self.fused else None               # fused graph network: adj once per env
             a, lp, h = self.actor(obs[lo:hi], node[lo:hi], adj_c, aid[lo:hi], rnn[lo:hi], masks[lo:hi],
                                   deterministic=self.deterministic, generator=self.generator, adj_env=adj_e)
-            v, hc = self.critic(None, node[lo:hi], adj_c, aid[lo:hi], rnn_c[lo:hi], masks[lo:hi], adj_env=adj_e)
+            cent, aid_c, cent_e = self._critic_inputs(t, lo, hi)
+            v, hc = self.critic(cent, node[lo:hi], adj_c, aid_c, rnn_c[lo:hi], masks[lo:hi], adj_env=adj_e, cent_env=cent_e)
             outs.append((v, a, lp, h, hc))
         if len(outs) == 1:
             return outs[0]
@@ -235,7 +249,8 @@ class RolloutCollector:
         B, N, E = b.n_rollout_threads, b.num_agents, b.num_entities
         M = B * N
         adj = b.adj_env[-1].unsqueeze(1).expand(B, N, E, E).reshape(M, E, E)
-        v, _ = self.critic(None, b.node_obs[-1].view(M, E, -1), adj, b.agent_id[-1].reshape(M, 1),
+        cent, aid, cent_e = self._critic_inputs(b.episode_length, 0, M)
+        v, _ = self.critic(cent, b.node_obs[-1].view(M, E, -1), adj, aid,
                            b.rnn_states_critic[-1].view(M, *b.rnn_states.shape[3:]), b.masks[-1].view(M, 1),
-                           adj_env=(b.adj_env[-1], N) if self.fused else None)
+                           adj_env=(b.adj_env[-1], N) if self.fused else None, cent_env=cent_e)
         b.compute_returns(v)

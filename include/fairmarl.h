@@ -369,6 +369,14 @@ int fm_gnn_supported(int32_t num_entities, int32_t node_feat_dim);
 int fm_gnn_mapping(int32_t num_entities, int32_t node_feat_dim);
 int fm_gnn_forward(int device, const FmGnnConfig* cfg, const float* weights, const float* node_obs, const float* adj,
                    const int32_t* agent_id, float* out, void* stream);
+/* The same forward with a multi-node gather as the epilogue (GNNBase with graph_aggr='node' and k node indices per graph,
+ * e.g. GR_Critic with critic_graph_aggr='node' gathering the N agent nodes through share_agent_id): the final states of
+ * the k nodes agent_id[m][0..k-1] side by side.  cfg as for fm_gnn_forward except that cfg->aggr must be 0;
+ *   agent_id  device int32 [num_graphs, k], 1 <= k <= num_entities (required)
+ *   out       device [num_graphs, k * 16];  out[m][16 i + c] = fm_gnn_forward's out for the one-node gather agent_id[m][i]
+ * Same mappings and weights as fm_gnn_forward; its kernels are the same code up to the epilogue. */
+int fm_gnn_gather(int device, const FmGnnConfig* cfg, int32_t k, const float* weights, const float* node_obs,
+                  const float* adj, const int32_t* agent_id, float* out, void* stream);
 
 /* Fused policy head behind the graph network: GR_Actor.forward / GR_Critic.forward after gnn_base
  * (onpolicy/algorithms/graph_actor_critic.py:150-178, :380-397): [obs | nbd] -> MLPBase (utils/mlp.py) -> one GRU step
@@ -394,6 +402,35 @@ int64_t fm_head_weight_floats(const FmHeadConfig* cfg);
 int fm_policy_head(int device, const FmHeadConfig* cfg, const float* weights, const float* obs, const float* nbd,
                    const float* rnn_in, const float* mask, const float* u, float* rnn_out, float* logp, int64_t* action,
                    float* value, void* stream);
+
+/* Fused critic head for wide inputs: GR_Critic.forward after gnn_base (graph_actor_critic.py:323-397) on
+ * x = [cent_obs | nbd] of D = cent_dim + nbd_dim features, 1 <= D <= 768: feature LayerNorm over all D inputs ->
+ * MLPBase -> one GRU step on h * mask + LayerNorm -> v_out.  It covers use_cent_obs (cent_obs = share_obs: the N agents'
+ * observations side by side, cent_dim = N * obs_dim) and critic_graph_aggr='node' (nbd = fm_gnn_gather's k = N node
+ * states, nbd_dim = N * 16), where fm_policy_head (obs_dim + 16 <= 32) does not.  hidden_size = 64, recurrent_N = 1.
+ *   weights  device, fm_critic_head_weight_floats() floats; Dp = D rounded up to a multiple of 32 (zero padded):
+ *              feature_norm gamma[Dp], beta[Dp]
+ *              fc1 [Dp / 4][64][4] (W^T k-quad interleaved), b[64], ln gamma[64], beta[64]
+ *              then exactly fm_policy_head's blob after its fc1 block: layers x { [16][64][4], b, gamma, beta },
+ *              recurrent: W_ih [16][192][4], W_hh [16][192][4], b_ih[192], b_hh[192], ln gamma[64], beta[64],
+ *              output W[8 rows][64] (row 0 = v_out, the rest zero), b[8]
+ *   cent_obs [num_rows / rows_per_env, cent_dim]: ONE row per env, read by its rows_per_env consecutive rows (NULL when
+ *            cent_dim == 0; num_rows must be a multiple of rows_per_env)
+ *   nbd [rows, nbd_dim], rnn_in [rows, 64], mask [rows] (recurrent), rnn_out [rows, 64] (recurrent), value [rows]
+ * fp32 on CUDA cores, deterministic and batch-invariant (the bits of a row do not depend on the batch around it). */
+typedef struct FmCriticHeadConfig {
+  int32_t num_rows;
+  int32_t cent_dim;         /* N * obs_dim with use_cent_obs, else 0 */
+  int32_t rows_per_env;     /* rows that share one cent_obs row (N) */
+  int32_t nbd_dim;          /* 16 (global pool) or k * 16 (fm_gnn_gather) */
+  int32_t layers;           /* layer_N: hidden layers after fc1, 0..2 */
+  int32_t recurrent;        /* use_recurrent_policy or use_naive_recurrent_policy */
+  int32_t feature_norm;     /* use_feature_normalization (the input LayerNorm) */
+  int32_t relu;             /* use_ReLU */
+} FmCriticHeadConfig;
+int64_t fm_critic_head_weight_floats(const FmCriticHeadConfig* cfg);
+int fm_critic_head(int device, const FmCriticHeadConfig* cfg, const float* weights, const float* cent_obs, const float* nbd,
+                   const float* rnn_in, const float* mask, float* rnn_out, float* value, void* stream);
 
 #ifdef __cplusplus
 }
