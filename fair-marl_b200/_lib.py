@@ -92,6 +92,35 @@ class FmCriticHeadConfig(C.Structure):
                 ("layers", C.c_int32), ("recurrent", C.c_int32), ("feature_norm", C.c_int32), ("relu", C.c_int32)]
 
 
+class FmReturnsConfig(C.Structure):
+    _fields_ = [("episode_length", C.c_int32), ("num_envs", C.c_int32), ("num_agents", C.c_int32), ("use_gae", C.c_int32),
+                ("use_proper_time_limits", C.c_int32), ("reserved_", C.c_int32), ("gamma", C.c_float), ("gamma_lambda", C.c_float)]
+
+
+MINIBATCH_MODES = {"feed_forward": 0, "recurrent": 1, "naive_recurrent": 2}     # FM_MINIBATCH_*
+ADV_WORKSPACE_DOUBLES = 768                                                     # FM_ADV_WORKSPACE_DOUBLES
+
+
+class FmMinibatchConfig(C.Structure):
+    _fields_ = [(name, C.c_int32) for name in (
+        "episode_length", "num_envs", "num_agents", "num_entities", "obs_dim", "node_feat_dim", "rnn_floats", "mode",
+        "num_mini_batch", "mini_batch_size", "data_chunk_length", "mini_batch")]
+
+
+BUFFER_SLAB_FIELDS = ("obs", "node_obs", "adj_env", "rnn_states", "rnn_states_critic", "actions", "action_log_probs",
+                      "value_preds", "returns", "masks", "active_masks", "advantages")
+MINIBATCH_FIELDS = ("share_obs", "obs", "node_obs", "adj", "agent_id", "share_agent_id", "rnn_states", "rnn_states_critic",
+                    "actions", "value_preds", "returns", "masks", "active_masks", "old_action_log_probs", "adv_targ")
+
+
+class FmBufferSlabs(C.Structure):
+    _fields_ = [(name, C.c_void_p) for name in BUFFER_SLAB_FIELDS]
+
+
+class FmMinibatch(C.Structure):
+    _fields_ = [(name, C.c_void_p) for name in MINIBATCH_FIELDS]
+
+
 class FairMarlError(RuntimeError):
     pass
 
@@ -161,6 +190,10 @@ def load():
         "fm_gnn_gather": ([C.c_int, C.POINTER(FmGnnConfig), i32, vp, vp, vp, vp, vp, vp], C.c_int),
         "fm_critic_head_weight_floats": ([C.POINTER(FmCriticHeadConfig)], i64),
         "fm_critic_head": ([C.c_int, C.POINTER(FmCriticHeadConfig), vp, vp, vp, vp, vp, vp, vp, vp], C.c_int),
+        "fm_buffer_returns": ([C.c_int, C.POINTER(FmReturnsConfig), vp, vp, vp, vp, vp, vp, vp, vp, vp], C.c_int),
+        "fm_buffer_advantages": ([C.c_int, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp], C.c_int),
+        "fm_buffer_minibatch": ([C.c_int, C.POINTER(FmMinibatchConfig), C.POINTER(FmBufferSlabs), vp, C.POINTER(FmMinibatch), vp],
+                                C.c_int),
     }
     for name, (argtypes, restype) in sig.items():
         fn = getattr(lib, name)          # AttributeError if the .so does not export the ABI
@@ -179,6 +212,7 @@ EXPORTED_SYMBOLS = (
     "fm_formation_get_state", "fm_formation_stats_enable", "fm_formation_stats_read", "fm_gnn_weight_floats", "fm_gnn_supported", "fm_gnn_mapping",
     "fm_gnn_forward",
     "fm_head_weight_floats", "fm_policy_head", "fm_gnn_gather", "fm_critic_head_weight_floats", "fm_critic_head",
+    "fm_buffer_returns", "fm_buffer_advantages", "fm_buffer_minibatch",
 )
 
 

@@ -12,7 +12,7 @@ from concurrent.futures import ThreadPoolExecutor
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _CSRC = os.path.join(_HERE, "csrc")
 _OBJ = os.path.join(_HERE, "build")
-SOURCES = ["fm_kernels.cu", "fm_aw.cu", "fm_roll.cu", "fm_formation.cu", "fm_form_image.cu", "fm_edges.cu", "fm_soa.cu", "fm_policy.cu", "fm_lsap.cu", "fm_abi.cu"]
+SOURCES = ["fm_kernels.cu", "fm_aw.cu", "fm_roll.cu", "fm_formation.cu", "fm_form_image.cu", "fm_edges.cu", "fm_soa.cu", "fm_policy.cu", "fm_lsap.cu", "fm_buffer.cu", "fm_abi.cu"]
 HEADERS = ["fm_device.cuh", "fm_launch.h", "fm_small.cuh", "fm_aw.cuh", "fm_form.cuh",
            os.path.join("..", "..", "include", "fairmarl.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

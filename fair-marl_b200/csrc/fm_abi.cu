@@ -1271,4 +1271,90 @@ int fm_critic_head(int device, const FmCriticHeadConfig* cfg, const float* weigh
   return FM_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Training side of the rollout buffer (fm_buffer.cu).
+static int buffer_shape(const char* fn, int32_t T, int32_t B, int32_t N) {
+  if (T < 1 || B < 1 || N < 1) return fail(FM_ERR_INVALID_ARG, "%s: episode_length %d / num_envs %d / num_agents %d (each >= 1)", fn, T, B, N);
+  if ((int64_t)T * B * N >= ((int64_t)1 << 31))
+    return fail(FM_ERR_INVALID_ARG, "%s: T * B * N = %lld samples (at most 2^31 - 1)", fn, (long long)T * B * N);
+  return FM_OK;
+}
+
+static bool norm_ok(const float* mean, const float* stdv) { return (mean == nullptr) == (stdv == nullptr); }
+
+int fm_buffer_returns(int device, const FmReturnsConfig* cfg, const float* next_value, float* value_preds, const float* rewards,
+                      const float* masks, const float* bad_masks, const float* norm_mean, const float* norm_std,
+                      float* returns, void* stream) {
+  if (!cfg || !next_value || !value_preds || !rewards || !masks || !returns || (cfg->use_proper_time_limits && !bad_masks))
+    return fail(FM_ERR_INVALID_ARG, "fm_buffer_returns: null argument");
+  if (!norm_ok(norm_mean, norm_std)) return fail(FM_ERR_INVALID_ARG, "fm_buffer_returns: norm_mean and norm_std are both given or both null");
+  if (int rc = buffer_shape("fm_buffer_returns", cfg->episode_length, cfg->num_envs, cfg->num_agents)) return rc;
+  if (int rc = use_device(device)) return rc;
+  FM_CUDA(fm::launch_buffer_returns(*cfg, next_value, value_preds, rewards, masks, bad_masks, norm_mean, norm_std, returns,
+                                    (cudaStream_t)stream));
+  return FM_OK;
+}
+
+int fm_buffer_advantages(int device, int32_t episode_length, int32_t num_envs, int32_t num_agents, const float* returns,
+                         const float* value_preds, const float* active_masks, const float* norm_mean, const float* norm_std,
+                         float* advantages, float* stats, double* workspace, void* stream) {
+  if (!returns || !value_preds || !active_masks || !advantages || !stats || !workspace)
+    return fail(FM_ERR_INVALID_ARG, "fm_buffer_advantages: null argument");
+  if (!norm_ok(norm_mean, norm_std)) return fail(FM_ERR_INVALID_ARG, "fm_buffer_advantages: norm_mean and norm_std are both given or both null");
+  if (int rc = buffer_shape("fm_buffer_advantages", episode_length, num_envs, num_agents)) return rc;
+  if (int rc = use_device(device)) return rc;
+  FM_CUDA(fm::launch_buffer_advantages((long long)episode_length * num_envs * num_agents, returns, value_preds, active_masks,
+                                       norm_mean, norm_std, advantages, stats, workspace, (cudaStream_t)stream));
+  return FM_OK;
+}
+
+int fm_buffer_minibatch(int device, const FmMinibatchConfig* cfg, const FmBufferSlabs* in, const int64_t* perm,
+                        const FmMinibatch* out, void* stream) {
+  if (!cfg || !in || !perm || !out) return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: null argument");
+  const void* const req[] = {in->obs, in->node_obs, in->adj_env, in->rnn_states, in->rnn_states_critic, in->actions,
+                             in->action_log_probs, in->value_preds, in->returns, in->masks, in->active_masks, in->advantages,
+                             out->share_obs, out->obs, out->node_obs, out->adj, out->agent_id, out->share_agent_id,
+                             out->rnn_states, out->rnn_states_critic, out->actions, out->value_preds, out->returns, out->masks,
+                             out->active_masks, out->old_action_log_probs, out->adv_targ};
+  for (const void* q : req)
+    if (!q) return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: null argument");
+  const int T = cfg->episode_length, B = cfg->num_envs, N = cfg->num_agents;
+  if (int rc = buffer_shape("fm_buffer_minibatch", T, B, N)) return rc;
+  if (cfg->num_entities < 1 || cfg->obs_dim < 1 || cfg->node_feat_dim < 1 || cfg->rnn_floats < 1)
+    return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: num_entities %d / obs_dim %d / node_feat_dim %d / rnn_floats %d (each >= 1)",
+                cfg->num_entities, cfg->obs_dim, cfg->node_feat_dim, cfg->rnn_floats);
+  const int64_t samples = (int64_t)T * B * N, K = cfg->num_mini_batch;
+  int64_t units, per, rows;                      // units: what the permutation ranges over
+  if (cfg->mode == FM_MINIBATCH_FEED_FORWARD) {
+    units = samples;
+    if (K < 1 || K > units) return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: num_mini_batch %lld for %lld samples", (long long)K, (long long)units);
+    if (cfg->mini_batch_size < 0 || (int64_t)cfg->mini_batch_size * K > units)
+      return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: %lld mini-batches of %d samples from %lld", (long long)K, cfg->mini_batch_size,
+                  (long long)units);
+    per = cfg->mini_batch_size ? cfg->mini_batch_size : units / K;
+    rows = per;
+  } else if (cfg->mode == FM_MINIBATCH_RECURRENT || cfg->mode == FM_MINIBATCH_NAIVE_RECURRENT) {
+    if (cfg->mini_batch_size != 0) return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: mini_batch_size is a feed-forward option");
+    const bool chunked = cfg->mode == FM_MINIBATCH_RECURRENT;
+    if (chunked && cfg->data_chunk_length < 1)
+      return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: data_chunk_length %d (>= 1)", cfg->data_chunk_length);
+    units = chunked ? samples / cfg->data_chunk_length : (int64_t)B * N;
+    if (K < 1 || K > units)
+      return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: num_mini_batch %lld for %lld %s", (long long)K, (long long)units,
+                  chunked ? "chunks" : "columns");
+    if (!chunked && units % K != 0)   // the reference yields another number of mini-batches, or raises IndexError mid-epoch
+      return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: %lld columns are not divisible by num_mini_batch %lld", (long long)units, (long long)K);
+    per = units / K;
+    rows = per * (chunked ? cfg->data_chunk_length : T);
+  } else {
+    return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: mode %d (0 feed-forward, 1 recurrent, 2 naive recurrent)", cfg->mode);
+  }
+  if (cfg->mini_batch < 0 || cfg->mini_batch >= K)
+    return fail(FM_ERR_INVALID_ARG, "fm_buffer_minibatch: mini_batch %d of %lld", cfg->mini_batch, (long long)K);
+  if (int rc = use_device(device)) return rc;
+  FM_CUDA(fm::launch_buffer_minibatch(*cfg, rows, per, (int)per, cfg->mini_batch * per, *in, (const long long*)perm, *out,
+                                      (cudaStream_t)stream));
+  return FM_OK;
+}
+
 }  // extern "C"

@@ -107,6 +107,16 @@ constexpr int CRITIC_HEAD_MAX_IN = 768;    // critic_head_kernel: input width ca
 int critic_head_weight_count(int in_dim, int layers, int recurrent);
 cudaError_t launch_critic_head(const FmCriticHeadConfig& c, const float* weights, const float* cent_obs, const float* nbd,
                                const float* rnn_in, const float* mask, float* rnn_out, float* value, cudaStream_t st);
+// training side of the rollout buffer (fm_buffer.cu); arguments checked by fm_abi.cu
+cudaError_t launch_buffer_returns(const FmReturnsConfig& c, const float* next_value, float* value_preds, const float* rewards,
+                                  const float* masks, const float* bad_masks, const float* norm_mean, const float* norm_std,
+                                  float* returns, cudaStream_t st);
+cudaError_t launch_buffer_advantages(long long n, const float* returns, const float* value_preds, const float* active_masks,
+                                     const float* norm_mean, const float* norm_std, float* advantages, float* stats,
+                                     double* workspace, cudaStream_t st);
+// rows output rows, rnn_rows of them with rnn states, per samples / chunks / columns per mini-batch, off = k * per
+cudaError_t launch_buffer_minibatch(const FmMinibatchConfig& c, long long rows, long long rnn_rows, int per, long long off,
+                                    const FmBufferSlabs& in, const long long* perm, const FmMinibatch& out, cudaStream_t st);
 int formation_max_agents();
 int set_error(int code, const char* fmt, ...);   // fm_last_error text (fm_abi.cu)
 }  // namespace fm

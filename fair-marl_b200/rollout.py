@@ -28,10 +28,12 @@ class DeviceRolloutBuffer:
 
     def __init__(self, episode_length: int, num_envs: int, num_agents: int, num_entities: int, obs_dim: int = 7,
                  node_feat_dim: int = 11, hidden_size: int = 64, recurrent_N: int = 1, action_dim: int = 5,
-                 gamma: float = 0.99, gae_lambda: float = 0.95, use_gae: bool = True, device: Any = "cuda"):
+                 gamma: float = 0.99, gae_lambda: float = 0.95, use_gae: bool = True, device: Any = "cuda",
+                 use_proper_time_limits: bool = False):
         T, B, N, E = int(episode_length), int(num_envs), int(num_agents), int(num_entities)
         self.episode_length, self.n_rollout_threads, self.num_agents, self.num_entities = T, B, N, E
         self.gamma, self.gae_lambda, self._use_gae = gamma, gae_lambda, use_gae
+        self._use_proper_time_limits = use_proper_time_limits
         self.device = torch.device(device)
         f32 = dict(dtype=torch.float32, device=self.device)
         self.obs = torch.zeros((T + 1, B, N, obs_dim), **f32)
@@ -52,6 +54,7 @@ class DeviceRolloutBuffer:
         self.bad_masks = torch.ones_like(self.masks)
         self.active_masks = torch.ones_like(self.masks)
         self.step = 0
+        self.advantage_stats: Optional[torch.Tensor] = None   # [2] (mean, std) of the last advantages() call
 
     # ---- views the reference materialises ------------------------------------------------------------------
     @property
@@ -106,21 +109,170 @@ class DeviceRolloutBuffer:
             x = getattr(self, name)
             x[0].copy_(x[-1])
 
-    def compute_returns(self, next_value: torch.Tensor) -> None:
-        """GAE / discounted returns without value normalisation and without proper time limits
-        (graph_buffer.py:314-341, the ``else`` branches)."""
+    def _norm_mean_std(self, value_normalizer) -> Optional[Tuple[torch.Tensor, torch.Tensor]]:
+        """(mean, std) as the reference's ``value_normalizer.denormalize`` applies them (x * sqrt(var) + mean):
+        ``ValueNorm.running_mean_var()`` or ``PopArt.debiased_mean_var()``, sqrt taken by torch in float32."""
+        if value_normalizer is None:
+            return None
+        if hasattr(value_normalizer, "running_mean_var"):
+            mean, var = value_normalizer.running_mean_var()
+        elif hasattr(value_normalizer, "debiased_mean_var"):
+            mean, var = value_normalizer.debiased_mean_var()
+        else:
+            raise TypeError("value_normalizer: expected the reference's ValueNorm (running_mean_var) or PopArt (debiased_mean_var)")
+        if mean.numel() != 1 or var.numel() != 1 or mean.dtype != torch.float32 or var.dtype != torch.float32:
+            raise ValueError("value_normalizer: a float32 normaliser of one value (input_shape 1) is expected")
+        mean, var = mean.detach().reshape(1), var.detach().reshape(1)
+        return mean.to(self.device), torch.sqrt(var).to(self.device)
+
+    def _stream(self) -> int:
+        return torch.cuda.current_stream(self.obs.device).cuda_stream
+
+    def compute_returns(self, next_value: torch.Tensor, value_normalizer=None) -> None:
+        """``GraphReplayBuffer.compute_returns`` (graph_buffer.py:285-366), every branch: GAE or discounted returns, with
+        or without ``use_proper_time_limits``, with or without a value normaliser (the reference's ValueNorm or PopArt:
+        the critic's values are then normalised and are denormalised here).  On a CUDA buffer this is one launch of
+        ``fm_buffer_returns``, bit for bit the reference's float32 loop; on a CPU buffer the torch loop below."""
+        norm = self._norm_mean_std(value_normalizer)
+        if self.obs.is_cuda:
+            import ctypes as C
+            from fair_marl_b200 import _lib
+            B, N = self.n_rollout_threads, self.num_agents
+            c = _lib.FmReturnsConfig(episode_length=self.episode_length, num_envs=B, num_agents=N, use_gae=int(self._use_gae),
+                                     use_proper_time_limits=int(self._use_proper_time_limits), gamma=float(self.gamma),
+                                     gamma_lambda=float(self.gamma * self.gae_lambda))
+            nv = next_value.detach().reshape(B * N).to(device=self.obs.device, dtype=torch.float32).contiguous()
+            _lib.check(_lib.load().fm_buffer_returns(
+                self.obs.device.index, C.byref(c), nv.data_ptr(), self.value_preds.data_ptr(), self.rewards.data_ptr(),
+                self.masks.data_ptr(), self.bad_masks.data_ptr(), norm[0].data_ptr() if norm else None,
+                norm[1].data_ptr() if norm else None, self.returns.data_ptr(), self._stream()), "fm_buffer_returns")
+            return
+        dv = (lambda x: x) if norm is None else (lambda x: x * norm[1] + norm[0])
         T = self.episode_length
         if self._use_gae:
             self.value_preds[-1] = next_value.view_as(self.value_preds[-1])
             gae = torch.zeros_like(self.value_preds[0])
             for t in reversed(range(T)):
-                delta = self.rewards[t] + self.gamma * self.value_preds[t + 1] * self.masks[t + 1] - self.value_preds[t]
+                delta = self.rewards[t] + self.gamma * dv(self.value_preds[t + 1]) * self.masks[t + 1] - dv(self.value_preds[t])
                 gae = delta + self.gamma * self.gae_lambda * self.masks[t + 1] * gae
-                self.returns[t] = gae + self.value_preds[t]
+                if self._use_proper_time_limits:
+                    gae = gae * self.bad_masks[t + 1]
+                self.returns[t] = gae + dv(self.value_preds[t])
         else:
             self.returns[-1] = next_value.view_as(self.returns[-1])
             for t in reversed(range(T)):
-                self.returns[t] = self.returns[t + 1] * self.gamma * self.masks[t + 1] + self.rewards[t]
+                if self._use_proper_time_limits:     # the reference denormalises in this branch only
+                    self.returns[t] = ((self.returns[t + 1] * self.gamma * self.masks[t + 1] + self.rewards[t]) * self.bad_masks[t + 1]
+                                       + (1 - self.bad_masks[t + 1]) * dv(self.value_preds[t]))
+                else:
+                    self.returns[t] = self.returns[t + 1] * self.gamma * self.masks[t + 1] + self.rewards[t]
+
+    # ---- the trainer's input (GR_MAPPO.train, graph_mappo.py:280-359) --------------------------------------------
+    def _require_cuda(self, what: str) -> None:
+        if not self.obs.is_cuda:
+            raise ValueError(f"DeviceRolloutBuffer.{what}: needs a CUDA buffer (fm_buffer.cu has no CPU path)")
+
+    def advantages(self, value_normalizer=None) -> torch.Tensor:
+        """The normalised advantages GR_MAPPO.train hands to the generators, [T, B, N, 1]: returns[:T] minus the
+        (denormalised) values, then (adv - mean) / (std + 1e-5) with the mean and population std over the entries whose
+        active_masks[:T] != 0 (np.nanmean / np.nanstd there; NaN when no entry is active).  Two launches of
+        ``fm_buffer_advantages``; the (mean, std) used are left in ``advantage_stats``."""
+        self._require_cuda("advantages")
+        from fair_marl_b200 import _lib
+        norm = self._norm_mean_std(value_normalizer)
+        T, B, N = self.episode_length, self.n_rollout_threads, self.num_agents
+        f32 = dict(dtype=torch.float32, device=self.obs.device)
+        adv = torch.empty((T, B, N, 1), **f32)
+        stats = torch.empty(2, **f32)
+        ws = torch.empty(_lib.ADV_WORKSPACE_DOUBLES, dtype=torch.float64, device=self.obs.device)
+        _lib.check(_lib.load().fm_buffer_advantages(
+            self.obs.device.index, T, B, N, self.returns.data_ptr(), self.value_preds.data_ptr(), self.active_masks.data_ptr(),
+            norm[0].data_ptr() if norm else None, norm[1].data_ptr() if norm else None, adv.data_ptr(), stats.data_ptr(),
+            ws.data_ptr(), self._stream()), "fm_buffer_advantages")
+        self.advantage_stats = stats
+        return adv
+
+    def feed_forward_generator(self, advantages: torch.Tensor, num_mini_batch: Optional[int] = None,
+                               mini_batch_size: Optional[int] = None, generator: Optional[torch.Generator] = None):
+        """``GraphReplayBuffer.feed_forward_generator``: num_mini_batch mini-batches of mini_batch_size (default
+        T B N // num_mini_batch) samples drawn without replacement over (t, b, n); the remainder is dropped."""
+        if num_mini_batch is None:
+            raise ValueError("feed_forward_generator: num_mini_batch is required (the reference slices range(num_mini_batch))")
+        return self._minibatches(advantages, "feed_forward", num_mini_batch, mini_batch_size or 0, 0, generator)
+
+    def recurrent_generator(self, advantages: torch.Tensor, num_mini_batch: int, data_chunk_length: int,
+                            generator: Optional[torch.Generator] = None):
+        """``GraphReplayBuffer.recurrent_generator``: chunks of data_chunk_length consecutive steps of one (env, agent)
+        column (flat over (b, n, t), so a chunk runs on into the next column when T % L != 0, as in the reference),
+        num_mini_batch mini-batches of chunks // num_mini_batch chunks, rows ordered [L, chunks]; rnn states at each
+        chunk's first step."""
+        return self._minibatches(advantages, "recurrent", num_mini_batch, 0, data_chunk_length, generator)
+
+    def naive_recurrent_generator(self, advantages: torch.Tensor, num_mini_batch: int,
+                                  generator: Optional[torch.Generator] = None):
+        """``GraphReplayBuffer.naive_recurrent_generator``: whole columns, B N // num_mini_batch per mini-batch (B N must
+        be divisible by num_mini_batch), rows ordered [T, columns]; rnn states at t = 0."""
+        return self._minibatches(advantages, "naive_recurrent", num_mini_batch, 0, 0, generator)
+
+    def _minibatches(self, advantages, mode, num_mini_batch, mini_batch_size, L, generator):
+        """Checks the arguments as ``fm_buffer_minibatch`` does (so a refusal raises here, before the epoch starts),
+        draws the epoch's permutation on the device and returns the generator of 16-tuples."""
+        self._require_cuda(mode + "_generator")
+        T, B, N = self.episode_length, self.n_rollout_threads, self.num_agents
+        if tuple(advantages.shape) != (T, B, N, 1) or advantages.dtype != torch.float32 or advantages.device != self.obs.device:
+            raise ValueError(f"advantages: float32 [{T}, {B}, {N}, 1] on {self.obs.device} expected")
+        K = int(num_mini_batch)
+        if mode == "feed_forward":
+            units = T * B * N
+            if mini_batch_size < 0 or mini_batch_size * K > units:
+                raise ValueError(f"feed_forward_generator: {K} mini-batches of {mini_batch_size} samples from {units}")
+        elif mode == "recurrent":
+            if L < 1:
+                raise ValueError(f"recurrent_generator: data_chunk_length {L} (>= 1)")
+            units = T * B * N // L
+        else:
+            units = B * N
+        if K < 1 or K > units:
+            raise ValueError(f"{mode}_generator: num_mini_batch {K} for {units} {dict(feed_forward='samples', recurrent='chunks', naive_recurrent='columns')[mode]}")
+        if mode == "naive_recurrent" and units % K:
+            raise ValueError(f"naive_recurrent_generator: {units} columns are not divisible by num_mini_batch {K} "
+                             "(the reference would yield another number of mini-batches or raise IndexError part-way through the epoch)")
+        if T * B * N >= 1 << 31:
+            raise ValueError(f"{mode}_generator: T * B * N = {T * B * N} samples (at most 2^31 - 1)")
+        per = mini_batch_size or units // K
+        rows = per * {"feed_forward": 1, "recurrent": L, "naive_recurrent": T}[mode]
+        perm = torch.randperm(units, device=self.obs.device, generator=generator)
+        return self._gather_epoch(advantages.contiguous(), perm, mode, K, mini_batch_size, L, per, rows)
+
+    def _gather_epoch(self, advantages, perm, mode, K, mini_batch_size, L, per, rows):
+        import ctypes as C
+        from fair_marl_b200 import _lib
+        T, B, N, E = self.episode_length, self.n_rollout_threads, self.num_agents, self.num_entities
+        D, F, A = self.obs.shape[-1], self.node_obs.shape[-1], self.available_actions.shape[-1]
+        rnn_shape = self.rnn_states.shape[3:]
+        c = _lib.FmMinibatchConfig(episode_length=T, num_envs=B, num_agents=N, num_entities=E, obs_dim=D, node_feat_dim=F,
+                                   rnn_floats=rnn_shape.numel(), mode=_lib.MINIBATCH_MODES[mode], num_mini_batch=K,
+                                   mini_batch_size=mini_batch_size, data_chunk_length=L)
+        src = {"obs": self.obs, "node_obs": self.node_obs, "adj_env": self.adj_env, "rnn_states": self.rnn_states,
+               "rnn_states_critic": self.rnn_states_critic, "actions": self.actions, "action_log_probs": self.action_log_probs,
+               "value_preds": self.value_preds, "returns": self.returns, "masks": self.masks,
+               "active_masks": self.active_masks, "advantages": advantages}
+        slabs = _lib.FmBufferSlabs(**{k: v.data_ptr() for k, v in src.items()})
+        dev = self.obs.device
+        f32, i32 = dict(dtype=torch.float32, device=dev), dict(dtype=torch.int32, device=dev)
+        available = self.available_actions[0, 0, :1].expand(rows, A)
+        for k in range(K):
+            out = {"share_obs": torch.empty((rows, N * D), **f32), "obs": torch.empty((rows, D), **f32),
+                   "node_obs": torch.empty((rows, E, F), **f32), "adj": torch.empty((rows, E, E), **f32),
+                   "agent_id": torch.empty((rows, 1), **i32), "share_agent_id": torch.empty((rows, N), **i32),
+                   "rnn_states": torch.empty((per, *rnn_shape), **f32), "rnn_states_critic": torch.empty((per, *rnn_shape), **f32)}
+            out.update({name: torch.empty((rows, 1), **f32) for name in
+                        ("actions", "value_preds", "returns", "masks", "active_masks", "old_action_log_probs", "adv_targ")})
+            c.mini_batch = k
+            mb = _lib.FmMinibatch(**{name: t.data_ptr() for name, t in out.items()})
+            _lib.check(_lib.load().fm_buffer_minibatch(dev.index, C.byref(c), C.byref(slabs), perm.data_ptr(), C.byref(mb),
+                                                       self._stream()), "fm_buffer_minibatch")
+            yield tuple(out[name] for name in _lib.MINIBATCH_FIELDS) + (available,)
 
 
 class RolloutCollector:
@@ -243,8 +395,10 @@ class RolloutCollector:
         self._graph = g                              # the capture itself does not execute: b.step is back at 0, slabs untouched
 
     @torch.no_grad()
-    def finish(self) -> None:
-        """``GMPERunner.compute`` (:490-506): bootstrap value of the last slab, then the returns."""
+    def finish(self, value_normalizer=None) -> None:
+        """``GMPERunner.compute`` (:490-506): bootstrap value of the last slab, then the returns.  Pass the trainer's
+        ``value_normalizer`` (ValueNorm / PopArt) when the critic is trained on normalised values (use_valuenorm, the
+        reference's default): the returns are then computed from the denormalised values, as the reference does."""
         b = self.buffer
         B, N, E = b.n_rollout_threads, b.num_agents, b.num_entities
         M = B * N
@@ -253,4 +407,4 @@ class RolloutCollector:
         v, _ = self.critic(cent, b.node_obs[-1].view(M, E, -1), adj, aid,
                            b.rnn_states_critic[-1].view(M, *b.rnn_states.shape[3:]), b.masks[-1].view(M, 1),
                            adj_env=(b.adj_env[-1], N) if self.fused else None, cent_env=cent_e)
-        b.compute_returns(v)
+        b.compute_returns(v, value_normalizer)

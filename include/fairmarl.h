@@ -432,6 +432,98 @@ int64_t fm_critic_head_weight_floats(const FmCriticHeadConfig* cfg);
 int fm_critic_head(int device, const FmCriticHeadConfig* cfg, const float* weights, const float* cent_obs, const float* nbd,
                    const float* rnn_in, const float* mask, float* rnn_out, float* value, void* stream);
 
+/* Training side of the device rollout buffer (fm_buffer.cu; fair-marl_b200/rollout.py DeviceRolloutBuffer): what
+ * GraphReplayBuffer.compute_returns, the advantage lines of GR_MAPPO.train and the buffer's three mini-batch generators
+ * compute (onpolicy/utils/graph_buffer.py, onpolicy/algorithms/graph_mappo.py).  Every field is a dense float32 array in
+ * the buffer's layout: slab t of a [T(+1), B, N] field starts at t * B * N.  fp32 on CUDA cores with each operation rounded
+ * on its own in the reference's order, deterministic, no atomics, no host synchronisation (graph-capturable).
+ * A value normaliser (ValueNorm / PopArt) enters as two device floats, norm_mean and norm_std = sqrt(var), which its
+ * denormalize applies as x * std + mean; both NULL means none.
+ * Refusals (FM_ERR_INVALID_ARG, before the device is touched): a null required pointer, a dimension < 1, T * B * N >= 2^31. */
+typedef struct FmReturnsConfig {
+  int32_t episode_length, num_envs, num_agents;
+  int32_t use_gae;
+  int32_t use_proper_time_limits;
+  int32_t reserved_;
+  float gamma;              /* float(gamma) */
+  float gamma_lambda;       /* float(gamma * gae_lambda), the product taken in double */
+} FmReturnsConfig;
+/* next_value [B, N] is stored into value_preds[T] (use_gae) or returns[T] (not), as the reference does, then for t =
+ * T-1 .. 0 returns[t] follows every branch of compute_returns.  value_preds, returns, masks, bad_masks: [T+1, B, N];
+ * rewards [T, B, N]; bad_masks is read only with use_proper_time_limits (may be NULL otherwise). */
+int fm_buffer_returns(int device, const FmReturnsConfig* cfg, const float* next_value, float* value_preds, const float* rewards,
+                      const float* masks, const float* bad_masks, const float* norm_mean, const float* norm_std,
+                      float* returns, void* stream);
+
+/* advantages[:T] = returns[:T] - denormalize(value_preds[:T]), then (adv - mean) / (std + 1e-5) with mean and the
+ * population std (ddof 0) of the entries whose active_masks[:T] != 0, accumulated in fp64 (Welford / Chan, fixed order)
+ * and rounded to float32; with no active entry both are NaN, as numpy's nanmean / nanstd give.
+ *   stats      device float[2]: mean, std as used
+ *   workspace  device double[FM_ADV_WORKSPACE_DOUBLES] (scratch; two launches) */
+#define FM_ADV_WORKSPACE_DOUBLES 768
+int fm_buffer_advantages(int device, int32_t episode_length, int32_t num_envs, int32_t num_agents, const float* returns,
+                         const float* value_preds, const float* active_masks, const float* norm_mean, const float* norm_std,
+                         float* advantages, float* stats, double* workspace, void* stream);
+
+/* One mini-batch of an epoch of GraphReplayBuffer.feed_forward_generator / recurrent_generator /
+ * naive_recurrent_generator in one launch, given the epoch's permutation (int64, as torch.randperm draws it):
+ *   feed-forward  samples i = (t B + b) N + n, perm over T B N; per = mini_batch_size or T B N / num_mini_batch;
+ *                 row j reads sample perm[k per + j]; rnn states of each row's own sample (per rows)
+ *   recurrent     f = (b N + n) T + t, chunks = T B N / L, per = chunks / num_mini_batch, perm over the chunks; row
+ *                 l per + c reads f = perm[k per + c] L + l (a chunk runs on into the next column when T % L != 0, as in
+ *                 the reference); rnn states at each chunk's first step (per rows)
+ *   naive         columns j = b N + n, per = B N / num_mini_batch (B N must divide), perm over B N; row t per + c reads
+ *                 column perm[k per + c] at time t; rnn states at t = 0 (per rows)
+ * share_obs is read from the env's obs row, adj from adj_env[t, b], agent_id / share_agent_id are synthesised from n.
+ * Refusals besides the common ones: mode outside 0..2, data_chunk_length < 1 (recurrent), num_mini_batch < 1 or more
+ * mini-batches than samples / chunks / columns, num_mini_batch * mini_batch_size > T B N, B N not divisible by
+ * num_mini_batch (naive: the reference would then yield another number of mini-batches, or raise IndexError part-way
+ * through the epoch), mini_batch outside 0..num_mini_batch-1. */
+enum { FM_MINIBATCH_FEED_FORWARD = 0, FM_MINIBATCH_RECURRENT = 1, FM_MINIBATCH_NAIVE_RECURRENT = 2 };
+typedef struct FmMinibatchConfig {
+  int32_t episode_length, num_envs, num_agents, num_entities;
+  int32_t obs_dim, node_feat_dim;
+  int32_t rnn_floats;       /* recurrent_N * hidden_size */
+  int32_t mode;             /* FM_MINIBATCH_* */
+  int32_t num_mini_batch;
+  int32_t mini_batch_size;  /* feed-forward: samples per mini-batch, 0 = T B N / num_mini_batch; must be 0 otherwise */
+  int32_t data_chunk_length;
+  int32_t mini_batch;       /* k: which mini-batch of the epoch */
+} FmMinibatchConfig;
+typedef struct FmBufferSlabs {         /* device pointers, all required */
+  const float* obs;                    /* [T+1, B, N, obs_dim] */
+  const float* node_obs;               /* [T+1, B, N, E, node_feat_dim] */
+  const float* adj_env;                /* [T+1, B, E, E] */
+  const float* rnn_states;             /* [T+1, B, N, rnn_floats] */
+  const float* rnn_states_critic;
+  const float* actions;                /* [T, B, N] */
+  const float* action_log_probs;       /* [T, B, N] */
+  const float* value_preds;            /* [T+1, B, N] */
+  const float* returns;
+  const float* masks;
+  const float* active_masks;
+  const float* advantages;             /* [T, B, N] */
+} FmBufferSlabs;
+typedef struct FmMinibatch {           /* device pointers, all required; R rows, R' = per rnn-state rows */
+  float* share_obs;                    /* [R, N * obs_dim] */
+  float* obs;                          /* [R, obs_dim] */
+  float* node_obs;                     /* [R, E, node_feat_dim] */
+  float* adj;                          /* [R, E, E] */
+  int32_t* agent_id;                   /* [R] */
+  int32_t* share_agent_id;             /* [R, N] */
+  float* rnn_states;                   /* [R', rnn_floats] */
+  float* rnn_states_critic;
+  float* actions;                      /* [R] each */
+  float* value_preds;
+  float* returns;
+  float* masks;
+  float* active_masks;
+  float* old_action_log_probs;
+  float* adv_targ;
+} FmMinibatch;
+int fm_buffer_minibatch(int device, const FmMinibatchConfig* cfg, const FmBufferSlabs* in, const int64_t* perm,
+                        const FmMinibatch* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
